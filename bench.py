@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            this repository's CUDA path
   python bench.py --impl reference [...]                          the reference's own CPU path (oracle/_ref)
+  python bench.py [...] --dump-outputs DIR                        also writes the last timed step's map to DIR (dump_map)
 
 Workload (BASELINE.json configs[2], the one north_star quotes its target on): synthetic 512^3 = 134 217 728 gas
 particles (recipe S1 of SURVEY.md 8(d): jittered lattice in a unit periodic box, seed 12345) projected onto a
@@ -40,8 +41,10 @@ WIN0 = 0.5            # parity / CPU windows start at map coordinate 0.5 on both
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline measurement (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the map the last one computed to DIR/mass_map.npy (see dump_map)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--n", type=int, default=512, help="lattice size (particles = n^3, all ranks together)")
     ap.add_argument("--npix", type=int, default=4096)
@@ -55,7 +58,30 @@ def parse():
     ap.add_argument("--sub", default="c5,c2,c4", help="which sub-records to run")
     ap.add_argument("--cpu-target-s", type=float, default=12.0)
     ap.add_argument("--c5-full-n", type=int, default=1024, help="lattice size of the full-size config-5 record (8 GPUs, or --sub c5full)")
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the map of this repository's CUDA path; it does not apply to --impl reference")
+    return args
+
+
+DUMP_BYTES = 32 << 20     # a larger map is dumped as a fixed sample of this many bytes of its pixels
+
+
+def dump_map(dirname, img):
+    """Write the float64 map `img` (device tensor) to DIR/mass_map.npy so that two builds run with the same arguments can be
+    compared pixel for pixel: the whole (nx, ny) map when it fits DUMP_BYTES, else the pixels at DUMP_BYTES / 8 flat indices
+    drawn without replacement by np.random.default_rng(0), in ascending order (the same pixels for the same map size)."""
+    import torch
+    flat = img.reshape(-1)
+    if flat.numel() * 8 > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_BYTES // 8, replace=False))
+        host = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    else:
+        host = img.cpu().numpy()
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "mass_map.npy"), host.astype(np.float64, copy=False))
 
 
 def hbm_peak():
@@ -614,6 +640,8 @@ def main():
     clocks = sampler.stop(m0, m1) if rank == 0 else None
     ms_per_step = float(ms.item()) / args.steps
     value = N / (ms_per_step * 1e-3)
+    if rank == 0 and args.dump_outputs:          # before the calls below overwrite `out` (rank 0 holds the reduced map)
+        dump_map(args.dump_outputs, out[0])
 
     # ---- parity of the map that was just timed (rank 0 holds the reduced map) against the CPU oracle, on a window
     parity = cpu = timed_crop = None

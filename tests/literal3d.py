@@ -65,3 +65,13 @@ def grid3d_literal(pos, h, prop, grid_size, lo, hi, kernel_func=None, shifts=((0
                     r = np.sqrt(r2[mask])
                     out[xi, yi, zi] = np.sum(An[mask] * kernel_func(r, Hn[mask]))
     return out
+
+
+def project2d_literal(pos, h, prop, npix, axis, bounds, kernel_func=None):
+    """the reference's 2-D pixel rule itself: grid3d_literal on a one-voxel-thick grid at z = 0, fed the particles'
+    in-plane coordinates (columns of CoordinateAxes.plane_columns) and z = 0, so that r2 = dx**2 + dy**2 + 0"""
+    a, b = {0: (1, 2), 1: (0, 2), 2: (0, 1)}[axis]
+    flat = np.zeros_like(pos)
+    flat[:, 0], flat[:, 1] = pos[:, a], pos[:, b]
+    x0, x1, y0, y1 = bounds
+    return grid3d_literal(flat, h, prop, (npix, npix, 1), (x0, y0, 0.0), (x1, y1, 1.0), kernel_func)[:, :, 0]

@@ -4,8 +4,8 @@ oracle/_ref is present.  Pins the extension's oracle on something other than its
 import numpy as np
 import pytest
 
-from conftest import rel_l2
-from literal3d import grid3d_literal, quartic_spline_numpy, reference_kernel
+from conftest import load_golden, rel_l2
+from literal3d import grid3d_literal, project2d_literal, quartic_spline_numpy, reference_kernel
 
 
 def cloud(seed, n):
@@ -22,6 +22,13 @@ def test_reference_kernel_is_the_numpy_restatement_of_kernels_pyx():
     r = rng.uniform(0, 2.5, 5000); h = rng.uniform(0.5, 1.5, 5000)
     k = reference_kernel()
     assert np.allclose(k(r, h), quartic_spline_numpy(r, h), rtol=1e-14, atol=0)
+    # without oracle/_ref, k is the restatement itself: pin it, with the literal 2-D pixel rule, on the reference's stored maps
+    for name in ("single_particle", "single_particle_axis0", "single_particle_axis1", "cloud_axis0", "cloud_axis1",
+                 "cloud_axis2", "cloud_tiny_and_huge_h"):
+        g = load_golden(name)
+        assert str(g["kernel"]) == "cubic_spline_3d"
+        lit = project2d_literal(g["pos"], g["h"], g["prop"], int(g["npix"]), int(g["axis"]), g["bounds"], quartic_spline_numpy)
+        assert np.array_equal(lit != 0, g["ref_map"] != 0) and rel_l2(lit, g["ref_map"]) < 1e-13
 
 
 @pytest.mark.parametrize("size,lo,hi", [((14, 14, 14), (0.0, 0.0, 0.0), (1.0, 1.0, 1.0)), ((9, 16, 12), (0.1, 0.0, 0.2), (0.9, 1.2, 0.8))])

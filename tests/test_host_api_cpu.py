@@ -69,15 +69,20 @@ def test_python_callable_kernels_are_tabulated_on_the_host():
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from astro_sph_tools_b200 import CoordinateAxes
-    from astro_sph_tools_b200.tools.projections import create_image, quartic_spline_kernel
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        create_image(np.zeros((4, 3)), np.ones(4), np.ones(4), (8, 8), 4, CoordinateAxes.Z, 0.0, 1.0, 0.0, 1.0)
-    with pytest.raises(RuntimeError, match="no CPU fallback"):
-        quartic_spline_kernel(np.ones(3), np.ones(3))
+    """run in a child interpreter that sees no CUDA device, so that the check also runs on a machine with a GPU"""
+    import subprocess
+    import sys
+    code = (f"import sys; sys.path.insert(0, {ROOT!r})\n"
+            "import numpy as np, pytest\n"
+            "from astro_sph_tools_b200 import CoordinateAxes\n"
+            "from astro_sph_tools_b200.tools.projections import create_image, quartic_spline_kernel\n"
+            "with pytest.raises(RuntimeError, match='no CPU fallback'):\n"
+            "    create_image(np.zeros((4, 3)), np.ones(4), np.ones(4), (8, 8), 4, CoordinateAxes.Z, 0.0, 1.0, 0.0, 1.0)\n"
+            "with pytest.raises(RuntimeError, match='no CPU fallback'):\n"
+            "    quartic_spline_kernel(np.ones(3), np.ones(3))\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr
 
 
 def test_coordinate_axes_mirror():
