@@ -44,16 +44,48 @@ struct P3 {
     // written by bin3_kernel for the blocks that have pairs or large-h entries, read by emit3_kernel (one enumeration there)
     uint32_t *pcount;                // pairs of particle i
     uint64_t *pmask;                 // bit m: image m is tiled, bit 27 + m: image m is on the large-h list
-    const int *wexp;                 // binary exponent E of the largest |prop * norm(h)| of the call + kExpBias3 (0: none); the
-                                     // brick path stores float32 weights relative to 2^E (see wexp3_kernel)
+    const int *wexp;                 // [2] largest binary exponent of prop * norm(h) over the particles that may take the brick
+                                     // path + kExpBias3, and kExpBias3 - the smallest (0: none); see wexp3_kernel
 };
 
 // The brick kernels work on float32 weights, the 2-D reference rules on float64 in any unit system (ADVICE r1: 1e48 or 1e-59
-// are legitimate weights).  Rec3 has no room for a per-particle exponent, so one pre-pass takes the largest binary exponent E
-// of prop * norm(h) over the call (16 bytes per particle: 0.05 ms at 256^3 against a 70 ms step); records hold
-// prop * norm(h) * 2^-E <= 1 (weights more than 2^126 below the largest flush to zero), bricks sum in those units and multiply
-// by 2^E in float64 when they write.  The direct deposits of few-voxel particles use the float64 weight as before.
+// are legitimate weights), and one call may mix weights hundreds of binary orders apart.  Rec3 has no room for a
+// per-particle exponent, so one pre-pass takes the largest and the smallest binary exponent of prop * norm(h) over the
+// particles that may take the brick path (16 bytes per particle: 0.05 ms at 256^3 against a 70 ms step; the direct deposits
+// of few-voxel particles use the float64 weight and take no part).  The weights are staged in exponent BANDS of kWeightBand
+// binary orders: band j holds prop * norm(h) * 2^-T_j for exponents T_j - kWeightBand < e <= T_j (T_0 = the largest,
+// T_j = T_0 - j kWeightBand; the last band takes everything below) and 0 otherwise, bricks sum in those units and multiply
+// by 2^T_j in float64 when they write.  A staged weight is at least 2^-kWeightBand, so even times a shape factor near the
+// support edge it stays a normal float.  Nearly every call spans fewer orders than one band: bin3_kernel stages it and
+// the bricks are summed once, as they always were; each further band rewrites the record weights from prop and h in
+// float64 (rec3_weights_kernel, O(n)) and sums the bricks again over the same sorted pairs.
 constexpr int kExpBias3 = 1 << 20;
+constexpr int kWeightBand = 100;
+
+// band j of the call from the two words of wexp3_kernel: exponents bot <= e <= hi are staged relative to 2^top (hi = top
+// except in band 0, which takes everything above as well)
+struct Band3 { int top, bot, hi; };
+__host__ __device__ __forceinline__ Band3 band3(int wmax, int wmin, int j)
+{
+    if (wmax <= 0) return { 0, -(1 << 30), 1 << 30 };             // no finite non-zero weight may take the brick path
+    const int emax = wmax - kExpBias3, emin = kExpBias3 - wmin, top = emax - j * kWeightBand;
+    return { top, top - kWeightBand < emin ? -(1 << 30) : top - kWeightBand + 1, j == 0 ? 1 << 30 : top };
+}
+__host__ __device__ __forceinline__ int n_bands3(int wmax, int wmin)
+{
+    return wmax <= 0 ? 1 : ((wmax - kExpBias3) - (kExpBias3 - wmin)) / kWeightBand + 1;
+}
+
+// float32 record weight of band b (0 outside it; 0, inf and NaN as they are)
+__device__ __forceinline__ float band_weight3(double w, Band3 b)
+{
+    if (w != 0.0 && fabs(w) < INFINITY) {
+        int ex;
+        frexp(w, &ex);
+        if (ex < b.bot || ex > b.hi) return 0.f;
+    }
+    return (float)scalbn(w, -b.top);
+}
 
 
 // periodic image shift along axis c of image m (0 when there is a single image).  Computed arithmetically: a table in
@@ -72,17 +104,39 @@ __device__ __forceinline__ double norm3(const P3 &p, double h)
     return p.norm_dim == 3 ? t * ih : t;
 }
 
+// wexp[0] = largest exponent + kExpBias3, wexp[1] = kExpBias3 - smallest exponent, over the particles that may get a record.
+// A particle whose support spans at most small_max_vox voxels even unclipped (at most floor(4h / d) + 1 samples per axis lie
+// within 2h) is deposited directly in every periodic image and is left out: a heavy or tiny-h particle deposited directly
+// must not push the brick path's weights into a lower band.
 __global__ void __launch_bounds__(256) wexp3_kernel(P3 p, int *__restrict__ wexp)
 {
-    int e = 0;                                                    // biased exponent, 0 = nothing seen
+    int emax = 0, emin = 0;                                       // biased, 0 = nothing seen
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < p.n; i += (int64_t)gridDim.x * blockDim.x) {
         const double h = p.h[i];
         if (!(h > 0.0 && 2.0 * h < INFINITY)) continue;
+        const double span = 4.0 * h * (1.0 + 1e-9);
+        double vox = 1.0;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) vox *= floor(span * p.ax[c].inv_d) + 1.0;
+        if (vox <= (double)p.small_max_vox) continue;
         const double c = p.prop[i] * norm3(p, h);
-        if (c != 0.0 && fabs(c) < INFINITY) { int ex; frexp(c, &ex); e = max(e, ex + kExpBias3); }
+        if (c != 0.0 && fabs(c) < INFINITY) {
+            int ex;
+            frexp(c, &ex);
+            emax = max(emax, ex + kExpBias3);
+            emin = max(emin, kExpBias3 - ex);
+        }
     }
-    e = __reduce_max_sync(0xffffffffu, e);
-    if ((threadIdx.x & 31) == 0 && e > 0) atomicMax(wexp, e);
+    emax = __reduce_max_sync(0xffffffffu, emax);
+    emin = __reduce_max_sync(0xffffffffu, emin);
+    if ((threadIdx.x & 31) == 0 && emax > 0) { atomicMax(wexp, emax); atomicMax(wexp + 1, emin); }
+}
+
+// record weights of band b for every particle (the entries of particles without a record are never read)
+__global__ void __launch_bounds__(256) rec3_weights_kernel(P3 p, Rec3 *__restrict__ rec, Band3 b)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < p.n) rec[i].c = band_weight3(p.prop[i] * norm3(p, p.h[i]), b);
 }
 
 template <int SHAPE>
@@ -147,8 +201,7 @@ __global__ void __launch_bounds__(kBin3Threads) bin3_kernel(P3 p, Rec3 *__restri
             Rec3 r;
             r.x = x0[0]; r.y = x0[1]; r.z = x0[2];
             r.inv_h = (float)(1.0 / h);
-            const int e = __ldg(p.wexp);
-            r.c = (float)scalbn(p.prop[i] * norm3(p, h), e > 0 ? kExpBias3 - e : 0);          // relative to 2^E
+            r.c = band_weight3(p.prop[i] * norm3(p, h), band3(__ldg(p.wexp), __ldg(p.wexp + 1), 0));     // band 0
             rec[i] = r;
         }
     }
@@ -288,7 +341,7 @@ struct Acc3 {
     ShapeTab tab;
     const uint32_t *seg_off;     // work items over the brick lists (work_items.cuh); ntiles = number of bricks
     int ntiles;
-    const int *wexp;             // the float32 weights are relative to 2^(wexp[0] - kExpBias3)
+    int etop;                    // the float32 weights are relative to 2^etop (the top of the current band)
 };
 
 // One CTA per work item of a brick (a whole brick list, or an interleaved share of a long one), four autonomous warps (no CTA barrier): warp w owns the 4x4x8 column (x,y quadrant) of the brick and
@@ -449,7 +502,7 @@ __global__ void __launch_bounds__(kAcc3Threads) brick_accum_kernel(Acc3 a)
     const int xi = X0 + xl, yi = Y0 + yl;
     if (xi < a.n[0] && yi < a.n[1]) {
         // the sums are in units of 2^E: two exact power-of-two factors (one could overflow at the ends of the exponent range)
-        const int eb = a.wexp[0], e = eb > 0 ? min(max(eb - kExpBias3, -2040), 2040) : 0, e1 = e / 2, e2 = e - e1;
+        const int e = min(max(a.etop, -2040), 2040), e1 = e / 2, e2 = e - e1;
         const double sc1 = __longlong_as_double((long long)(e1 + 1023) << 52), sc2 = __longlong_as_double((long long)(e2 + 1023) << 52);
         double *row = a.out + ((size_t)xi * a.n[1] + yi) * a.n[2];
 #pragma unroll
@@ -642,6 +695,7 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
     AST_CUDA_TRY(cudaMemsetAsync(L.wexp, 0, 2 * sizeof(int), s));
     tk.end();
     uint64_t totals[2] = { 0, 0 };
+    int wexp[2] = { 0, 0 };
     if (p->n > 0) {
         tk.begin(0);
         {
@@ -663,6 +717,7 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
         AST_CUDA_TRY(cudaGetLastError());
         AST_CUDA_TRY(cudaMemcpyAsync(&totals[0], L.block_pairs + L.nb, sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
         AST_CUDA_TRY(cudaMemcpyAsync(&totals[1], L.block_huge + L.nb, sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        AST_CUDA_TRY(cudaMemcpyAsync(wexp, L.wexp, sizeof wexp, cudaMemcpyDeviceToHost, s));
         AST_CUDA_TRY(cudaStreamSynchronize(s));
     }
     const uint64_t T = totals[0], H = totals[1];
@@ -688,8 +743,9 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
         c.img_shift = a.img_shift;
         c.n_img = a.n_img;
         c.tab = a.tab;
-        c.wexp = L.wexp;
         c.n_huge = 0u;
+        const int n_bands = n_bands3(wexp[0], wexp[1]);
+        int rec_band = 0;                                           // the band whose weights the records hold (bin3_kernel: 0)
         for (int k = 0; k < 3; ++k) c.box[k] = a.box[k];
         static const int sm_count = [] { int dev = 0, n = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); return n; }();
         int64_t round_no = 0;
@@ -744,11 +800,20 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
                 AST_CUDA_TRY(scan_exclusive<uint32_t>(L.seg_off, L.nbricks + 1, L.seg_tmp, nullptr, s, &nls));
                 const int64_t max_items = L.nbricks + nw / (int64_t)seg_target;
                 tk.begin(5);
-                if (a.shape == SHAPE_CUBIC) brick_accum_kernel<SHAPE_CUBIC><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
-                else if (a.shape == SHAPE_WENDLAND) brick_accum_kernel<SHAPE_WENDLAND><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
-                else brick_accum_kernel<SHAPE_TABLE><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
+                for (int j = 0; j < n_bands; ++j) {
+                    const Band3 b = band3(wexp[0], wexp[1], j);
+                    if (j != rec_band) {
+                        rec3_weights_kernel<<<(unsigned)((p->n + 255) / 256), 256, 0, s>>>(a, L.rec, b);
+                        rec_band = j;
+                        st.n_launches += 1;
+                    }
+                    c.etop = b.top;
+                    if (a.shape == SHAPE_CUBIC) brick_accum_kernel<SHAPE_CUBIC><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
+                    else if (a.shape == SHAPE_WENDLAND) brick_accum_kernel<SHAPE_WENDLAND><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
+                    else brick_accum_kernel<SHAPE_TABLE><<<(unsigned)max_items, kAcc3Threads, 0, s>>>(c);
+                }
                 tk.end();
-                st.n_launches += 6 + nl + nls;
+                st.n_launches += 5 + n_bands + nl + nls;
                 AST_CUDA_TRY(cudaGetLastError());
             }
         }

@@ -48,13 +48,21 @@ struct __align__(32) Rec {
 static_assert(sizeof(Rec) == 32, "record is one 32-byte sector");
 
 // The tile kernels work on float32 weights, the reference on float64 in any unit system (a luminosity in erg/s times
-// 1/(pi h^3) with h in Mpc is ~1e48; Msun masses with lengths in cm ~1e-59: both outside float32).  A weight is therefore
-// stored as a float32 mantissa and its own binary exponent; K1 also takes the maximum exponent E_k of every weight field
-// over the call, the staged per-pair weight is mantissa * 2^(e - E_k) <= 1 (weights more than 2^126 below the largest one of
-// the call flush to zero), the tile sums are formed in those units and multiplied by 2^E_k in float64 when they are added to
-// the map.  Powers of two only: no rounding is added anywhere.
+// 1/(pi h^3) with h in Mpc is ~1e48; Msun masses with lengths in cm ~1e-59: both outside float32), and one call may mix
+// weights hundreds of binary orders apart (an ion column density: ion fractions of 1e-40 next to 1).  A weight is therefore
+// stored as a float32 mantissa and its own binary exponent; K1 also takes the largest and the smallest exponent of every
+// weight field over the particles that have records.  The pair weights are staged in exponent BANDS of kWeightBand binary
+// orders: band j of field k stages mantissa * 2^(e - T_j) for T_j - kWeightBand < e <= T_j (T_0 = the largest exponent,
+// T_j = T_0 - j kWeightBand) and 0 otherwise, the tile sums are formed in those units and multiplied by 2^T_j in float64
+// when they are added to the map.  A staged weight is then at least 2^-kWeightBand, so even times a shape factor near the
+// support edge it stays a normal float.  Nearly every call spans fewer orders than one band: it stages and accumulates
+// once, as it always did; each further band repeats the staging and the accumulate kernel over the same sorted pairs.
+// Powers of two only: no rounding is added anywhere.
 constexpr int kZeroExp = -32768;
-constexpr int kExpBias = 1 << 20;       // stored maximum exponent = exponent + kExpBias > 0, so a zeroed control block means "none"
+constexpr int kExpBias = 1 << 20;       // stored exponents are exponent + kExpBias (maximum) and kExpBias - exponent (minimum),
+                                        // both > 0, so a zeroed control block means "none"
+constexpr int kWeightBand = 100;
+constexpr int kExpWords = (AST_MAX_PROPS * (int)sizeof(int) + 7) / 8;    // 64-bit words of one exponent array in the control block
 __device__ __forceinline__ void split_weight(double c, float &m, int &e)
 {
     if (c == 0.0) { m = 0.f; e = kZeroExp; return; }
@@ -86,6 +94,7 @@ struct P2 {
                                         // 64 tiles) and tx0 | ty0 << 24 | rows << 48
     int *wexp;                          // [AST_MAX_PROPS] maximum weight exponent of the call + kExpBias (atomicMax by K1; 0 = no
                                         // weight seen), see split_weight
+    int *wmin;                          // [AST_MAX_PROPS] kExpBias - minimum weight exponent of the call (atomicMax by K1)
     unsigned long long *totals;         // [2] pairs and large-h entries of the call (atomicAdd by the K1 blocks that have any)
 };
 
@@ -252,9 +261,12 @@ __device__ __forceinline__ void bin_particle(const P2 &p, int64_t i, double pa0,
             r.c[k] = 0.f;
             if (k < NP) split_weight(coef[k < NP ? k : 0], r.c[k], e);
             r.e[k] = (int16_t)e;
-            // running maximum of the call: a plain (possibly stale) read settles it for all but the first few warps, the
-            // atomic only runs when this particle would raise it
-            if (k < NP && e != kZeroExp && e + kExpBias > __ldcg(p.wexp + k)) atomicMax(p.wexp + k, e + kExpBias);
+            // running maximum and minimum of the call: a plain (possibly stale) read settles them for all but the first few
+            // warps, the atomic only runs when this particle would move one
+            if (k < NP && e != kZeroExp) {
+                if (e + kExpBias > __ldcg(p.wexp + k)) atomicMax(p.wexp + k, e + kExpBias);
+                if (kExpBias - e > __ldcg(p.wmin + k)) atomicMax(p.wmin + k, kExpBias - e);
+            }
         }
         rec[i] = r;
     }
@@ -645,8 +657,15 @@ struct Acc {
     uint32_t seg_target;          // target list entries per segment
     uint32_t n_huge;              // always 0 here (work_items.cuh is shared with the 3-D grid, which still walks a global list)
     int ntiles;
-    const int *wexp;              // [AST_MAX_PROPS] the float32 weights are relative to 2^wexp[k] (see split_weight)
+    int etop[AST_MAX_PROPS];      // exponent band of the staged weights (see split_weight): exponents etop - kWeightBand < e <=
+    int ebot[AST_MAX_PROPS];      // etop (ebot <= e <= etop, ebot = kZeroExp in the lowest band) are staged relative to 2^etop
 };
+
+// pair weight of band [ebot, etop] relative to 2^etop, 0 outside it
+__device__ __forceinline__ float stage_weight(float c, int e, int etop, int ebot)
+{
+    return (e >= ebot && e <= etop) ? ldexpf(c, max(e - etop, -300)) : 0.f;
+}
 
 // K5: first / one-past-last sorted pair of every tile (arrays pre-zeroed), and every sorted pair is turned into the two things the accumulate kernel
 // needs -- tile-relative float32 coordinates {fx, fy, sx, sy} and the weights -- ONCE, here.  The accumulate kernel used to do
@@ -669,9 +688,9 @@ __global__ void __launch_bounds__(256) pair_record_kernel(Acc a, int64_t n, uint
     const float fy = (float)((r.pb + image_shift_b(a.n_img, a.box_b, (int)m) - a.y_min) * a.inv_dy - oy);
     const float cscale = SHAPE == SHAPE_CUBIC ? 2.0f : 1.0f;
     pp[i] = make_float4(fx, fy, (float)a.dx * r.inv_h, (float)a.dy * r.inv_h);
-    // weights relative to 2^E_k (E_k = largest exponent of the call): mantissa * 2^(e - E_k), at most 1 in magnitude
-    const float w0 = ldexpf(r.c[0], max((int)r.e[0] - (a.wexp[0] - kExpBias), -300));
-    const float w1 = NP > 1 ? ldexpf(r.c[1], max((int)r.e[1] - (a.wexp[1] - kExpBias), -300)) : 0.f;
+    // weights of the current band relative to its top 2^etop_k: mantissa * 2^(e - etop_k), at most 1 in magnitude
+    const float w0 = stage_weight(r.c[0], r.e[0], a.etop[0], a.ebot[0]);
+    const float w1 = NP > 1 ? stage_weight(r.c[1], r.e[1], a.etop[1], a.ebot[1]) : 0.f;
     pc[i] = make_float2(cscale * w0, cscale * w1);
 }
 
@@ -844,11 +863,11 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
                 for (int jj = 0; jj < NPIX; ++jj) { acc64[k][jj] += (double)acc[k][jj]; acc[k][jj] = 0.f; }
         }
     }
-    // the sums are in units of 2^E_k: two exact power-of-two factors (E_k spans -1073 .. 1024, one factor could overflow)
+    // the sums are in units of 2^etop_k: two exact power-of-two factors (etop_k spans -1073 .. 1024, one factor could overflow)
     double sc1[NP], sc2[NP];
 #pragma unroll
     for (int k = 0; k < NP; ++k) {
-        const int e = min(max(a.wexp[k] - kExpBias, -2040), 2040), e1 = e / 2, e2 = e - e1;
+        const int e = min(max(a.etop[k], -2040), 2040), e1 = e / 2, e2 = e - e1;
         sc1[k] = __longlong_as_double((long long)(e1 + 1023) << 52);
         sc2[k] = __longlong_as_double((long long)(e2 + 1023) << 52);
     }
@@ -934,9 +953,9 @@ struct Layout2 {
     uint64_t *pairs_a, *pairs_b, *huge, *hoff, *hoff_tmp;
     uint32_t *pcount, *pmask;
     uint64_t *ptmask, *ptorg;
-    unsigned long long *ctrl;   // control block: totals[2], heavy block count, then the biased weight exponents (int[AST_MAX_PROPS]);
-                                // zeroed per call
-    int *wexp;
+    unsigned long long *ctrl;   // control block: totals[2], heavy block count, then the biased maximum and minimum weight exponents
+                                // (int[AST_MAX_PROPS] each, kExpWords words each); zeroed per call
+    int *wexp, *wmin;
     uint8_t *block_heavy;       // nb flags written by K0: the block holds particles K1 has to classify
     PresortBuffers pre;         // only with AST_FLAG_ORDER_AUTO / _ALWAYS
     RoundSet set;
@@ -980,8 +999,9 @@ static Layout2 layout2(const ast_project2d_params *p, void *ws)
     L.pmask = c.take<uint32_t>(p->n > 0 ? p->n : 1);
     L.ptmask = c.take<uint64_t>(p->n > 0 ? p->n : 1);
     L.ptorg = c.take<uint64_t>(p->n > 0 ? p->n : 1);
-    L.ctrl = c.take<unsigned long long>(3 + (AST_MAX_PROPS * sizeof(int) + 7) / 8);
+    L.ctrl = c.take<unsigned long long>(3 + 2 * kExpWords);
     L.wexp = reinterpret_cast<int *>(L.ctrl ? L.ctrl + 3 : nullptr);
+    L.wmin = reinterpret_cast<int *>(L.ctrl ? L.ctrl + 3 + kExpWords : nullptr);
     L.block_heavy = c.take<uint8_t>(L.nb + 1);
     L.pairs_a = c.take<uint64_t>(L.win);
     L.pairs_b = c.take<uint64_t>(L.win);
@@ -1038,7 +1058,7 @@ static P2 make_p2(const ast_project2d_params *p, const double *pos, const double
     a.small_max_px = p->small_max_px >= 0 ? p->small_max_px : kDefaultSmallMaxPx;
     a.huge_min_tiles = p->huge_min_tiles >= 0 ? p->huge_min_tiles : kDefaultHugeMinTiles;
     a.map_stride = (size_t)p->nx * (size_t)p->ny;
-    a.pcount = nullptr; a.pmask = nullptr; a.wexp = nullptr; a.totals = nullptr; a.ptmask = nullptr; a.ptorg = nullptr;
+    a.pcount = nullptr; a.pmask = nullptr; a.wexp = nullptr; a.wmin = nullptr; a.totals = nullptr; a.ptmask = nullptr; a.ptorg = nullptr;
     return a;
 }
 
@@ -1072,18 +1092,47 @@ struct Run2 {
     Acc c;
     cudaStream_t s;
     float2 *pc;                    // staged weights of the current round
+    const uint64_t *sorted;        // sorted pairs of the current round
+    int n_bands;                   // exponent bands of the call (1 unless the weights of one field span more than kWeightBand)
+    int emax[AST_MAX_PROPS], nbk[AST_MAX_PROPS];   // largest weight exponent and number of bands per field
     ast_project2d_stats st;
     StageTimer *tk;
     int sm_count;
 };
 
+// band j of every field into R.c (see split_weight); a field with fewer bands stages zeros from its last band on
+static void set_band(Run2 &R, int j)
+{
+    for (int k = 0; k < AST_MAX_PROPS; ++k) {
+        const int top = R.emax[k] - j * kWeightBand;
+        R.c.etop[k] = j < R.nbk[k] ? top : R.emax[k];
+        R.c.ebot[k] = j < R.nbk[k] ? (j + 1 == R.nbk[k] ? kZeroExp : top - kWeightBand + 1) : R.emax[k] + 1;
+    }
+}
+
+// K5 over the sorted pairs of the current round: tile ranges, coordinates and the weights of the band in R.c
+static void launch_pair_records(Run2 &R, int64_t nw)
+{
+    const RoundSet &S = R.L.set;
+    Acc c = R.c;
+    c.sorted = R.sorted;
+    const unsigned nbk = (unsigned)((nw + 255) / 256);
+    cudaStream_t q = R.s;
+#define AST_LAUNCH_PR(SH) do { if (R.p->n_prop == 1) pair_record_kernel<SH, 1><<<nbk, 256, 0, q>>>(c, nw, S.tbeg, S.tend, S.pp, R.pc); \
+                               else pair_record_kernel<SH, 2><<<nbk, 256, 0, q>>>(c, nw, S.tbeg, S.tend, S.pp, R.pc); } while (0)
+    if (R.a.shape == SHAPE_CUBIC) AST_LAUNCH_PR(SHAPE_CUBIC);
+    else if (R.a.shape == SHAPE_WENDLAND) AST_LAUNCH_PR(SHAPE_WENDLAND);
+    else AST_LAUNCH_PR(SHAPE_TABLE);
+#undef AST_LAUNCH_PR
+    R.st.n_launches += 1;
+}
+
 // index work of one round: pairs [w0, w1) of the combined emit order -- tiled pairs [0, T), then the pairs of the current
 // large-h window [base, base + HP): emit, stable sort by tile key, pair records, tile ranges, work items.
 static int prep_round(Run2 &R, uint64_t w0, uint64_t w1, uint64_t T, uint64_t base, uint64_t HP, uint32_t n_hent, uint32_t *seg_target)
 {
-    const ast_project2d_params *p = R.p;
     const Layout2 &L = R.L;
-    RoundSet S = L.set;
+    const RoundSet &S = L.set;
     cudaStream_t q = R.s;
     const int64_t nw = (int64_t)(w1 - w0);
     R.tk->begin(2);
@@ -1105,21 +1154,14 @@ static int prep_round(Run2 &R, uint64_t w0, uint64_t w1, uint64_t T, uint64_t ba
     R.tk->begin(4);
     AST_CUDA_TRY(cudaMemsetAsync(S.tbeg, 0, sizeof(uint32_t) * L.ntiles, q));
     AST_CUDA_TRY(cudaMemsetAsync(S.tend, 0, sizeof(uint32_t) * L.ntiles, q));
-    Acc c = R.c;
-    c.sorted = in_b ? L.pairs_b : L.pairs_a;
-    S.pc = R.pc = reinterpret_cast<float2 *>(in_b ? L.pairs_a : L.pairs_b);      // 8 bytes per pair, like the pairs
-    const unsigned nbk = (unsigned)((nw + 255) / 256);
-#define AST_LAUNCH_PR(SH) do { if (p->n_prop == 1) pair_record_kernel<SH, 1><<<nbk, 256, 0, q>>>(c, nw, S.tbeg, S.tend, S.pp, S.pc); \
-                               else pair_record_kernel<SH, 2><<<nbk, 256, 0, q>>>(c, nw, S.tbeg, S.tend, S.pp, S.pc); } while (0)
-    if (R.a.shape == SHAPE_CUBIC) AST_LAUNCH_PR(SHAPE_CUBIC);
-    else if (R.a.shape == SHAPE_WENDLAND) AST_LAUNCH_PR(SHAPE_WENDLAND);
-    else AST_LAUNCH_PR(SHAPE_TABLE);
-#undef AST_LAUNCH_PR
+    R.sorted = in_b ? L.pairs_b : L.pairs_a;
+    R.pc = reinterpret_cast<float2 *>(in_b ? L.pairs_a : L.pairs_b);      // 8 bytes per pair, like the pairs
+    launch_pair_records(R, nw);
     *seg_target = segment_target(nw, (int64_t)R.sm_count * 4);
     tile_segments_kernel<<<(unsigned)((L.ntiles + 1 + 255) / 256), 256, 0, q>>>(S.tbeg, S.tend, 0u, *seg_target, (int)L.ntiles, S.seg_off);
     nl = 0;
     AST_CUDA_TRY(scan_exclusive<uint32_t>(S.seg_off, L.ntiles + 1, S.seg_tmp, nullptr, q, &nl));
-    R.st.n_launches += 2 + nl;
+    R.st.n_launches += 1 + nl;
     R.tk->end();
     AST_CUDA_TRY(cudaGetLastError());
     return AST_OK;
@@ -1194,13 +1236,15 @@ extern "C" int ast_project2d(const ast_project2d_params *p, const double *pos, c
     }
     R.a = make_p2(p, pos, h, prop, out);
     P2 &a = R.a;
-    a.pcount = L.pcount; a.pmask = L.pmask; a.wexp = L.wexp; a.totals = L.ctrl; a.ptmask = L.ptmask; a.ptorg = L.ptorg;
+    a.pcount = L.pcount; a.pmask = L.pmask; a.wexp = L.wexp; a.wmin = L.wmin; a.totals = L.ctrl; a.ptmask = L.ptmask; a.ptorg = L.ptorg;
     { int dev = 0; R.sm_count = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&R.sm_count, cudaDevAttrMultiProcessorCount, dev); }
 
     if (!(p->flags & AST_FLAG_ACCUMULATE)) AST_CUDA_TRY(cudaMemsetAsync(out, 0, sizeof(double) * a.map_stride * p->n_prop, s));
-    AST_CUDA_TRY(cudaMemsetAsync(L.ctrl, 0, sizeof(unsigned long long) * 3 + sizeof(int) * AST_MAX_PROPS, s));     // totals, heavy count, exponents
+    AST_CUDA_TRY(cudaMemsetAsync(L.ctrl, 0, sizeof(unsigned long long) * (3 + 2 * kExpWords), s));     // totals, heavy count, exponents
     tk.end();
     uint64_t totals[2] = { 0, 0 };
+    unsigned long long ctl[3 + 2 * kExpWords];
+    memset(ctl, 0, sizeof ctl);
     if (p->n > 0) {
         tk.begin(0);
         {
@@ -1276,9 +1320,11 @@ extern "C" int ast_project2d(const ast_project2d_params *p, const double *pos, c
         tk.end();
         AST_CUDA_TRY(cudaGetLastError());
         // the K1 blocks that have pairs or large-h entries added them to the control block: when nothing needs the tile path
-        // (the HBM-bound regime: every particle was deposited by K1) the call ends here, without the scan
-        AST_CUDA_TRY(cudaMemcpyAsync(totals, L.ctrl, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        // (the HBM-bound regime: every particle was deposited by K1) the call ends here, without the scan.  The weight
+        // exponents come with the same copy: they decide the bands.
+        AST_CUDA_TRY(cudaMemcpyAsync(ctl, L.ctrl, sizeof ctl, cudaMemcpyDeviceToHost, s));
         AST_CUDA_TRY(cudaStreamSynchronize(s));
+        totals[0] = ctl[0]; totals[1] = ctl[1];
         if (totals[0] + totals[1] > 0) {
             tk.begin(1);
             // entries 0..nb-1 were written by the binning kernels; the sentinel entry nb becomes the total
@@ -1307,7 +1353,18 @@ extern "C" int ast_project2d(const ast_project2d_params *p, const double *pos, c
         c.x_min = a.ax.vmin; c.y_min = a.ay.vmin; c.dx = a.ax.d; c.dy = a.ay.d; c.inv_dx = a.ax.inv_d; c.inv_dy = a.ay.inv_d;
         c.nx = p->nx; c.ny = p->ny; c.ntx = a.ntx; c.nty = a.nty; c.img_shift = a.img_shift;
         c.n_img = a.n_img; c.box_a = a.box_a; c.box_b = a.box_b; c.tab = a.tab;
-        c.map_stride = a.map_stride; c.ntiles = (int)L.ntiles; c.wexp = L.wexp; c.n_huge = 0u;
+        c.map_stride = a.map_stride; c.ntiles = (int)L.ntiles; c.n_huge = 0u;
+        int wexp[AST_MAX_PROPS], wmin[AST_MAX_PROPS];
+        memcpy(wexp, ctl + 3, sizeof wexp);
+        memcpy(wmin, ctl + 3 + kExpWords, sizeof wmin);
+        R.n_bands = 1;
+        for (int k = 0; k < AST_MAX_PROPS; ++k) {
+            const bool any = k < p->n_prop && wexp[k] > 0;        // 0: no non-zero weight in this field
+            R.emax[k] = wexp[k] - kExpBias;
+            R.nbk[k] = any ? (R.emax[k] - (kExpBias - wmin[k])) / kWeightBand + 1 : 1;
+            if (R.nbk[k] > R.n_bands) R.n_bands = R.nbk[k];
+        }
+        set_band(R, 0);
 
         int rc2 = AST_OK;
         int64_t round_no = 0;
@@ -1342,9 +1399,15 @@ extern "C" int ast_project2d(const ast_project2d_params *p, const double *pos, c
             for (uint64_t r = 0; r * per_round < total && rc2 == AST_OK; ++r, ++round_no) {
                 const uint64_t w0 = r * per_round, w1 = (w0 + per_round < total) ? w0 + per_round : total;
                 uint32_t seg_target = 1024;
+                if (R.n_bands > 1) set_band(R, 0);
                 rc2 = prep_round(R, w0, w1, hw == 0 ? T : 0, base, HP, n_hent, &seg_target);
                 if (rc2) break;
                 rc2 = accumulate_round(R, (int64_t)(w1 - w0), seg_target);
+                for (int j = 1; j < R.n_bands && rc2 == AST_OK; ++j) {       // the further bands over the same sorted pairs
+                    set_band(R, j);
+                    launch_pair_records(R, (int64_t)(w1 - w0));
+                    rc2 = accumulate_round(R, (int64_t)(w1 - w0), seg_target);
+                }
             }
         }
         st.n_rounds = round_no;

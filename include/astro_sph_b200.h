@@ -109,8 +109,9 @@ int ast_project2d_workspace_bytes(const ast_project2d_params *p, size_t *bytes /
  * the call ends there) and once more per large-h window.  pair_capacity and huge_capacity are windows: no value > 0 can
  * make the call fail, and nothing is deposited twice.  The one AST_EWORKSPACE that can be returned AFTER `out` has been
  * written to (the direct deposits of the binning kernel) is pair_capacity <= 0 with particles that need the tile path.
- * Weights are float64 and keep float64 range (the tile path stores mantissa + exponent, sums in units of the call's largest
- * power of two, scales back in float64). */
+ * Weights are float64 and keep float64 range, also when one call mixes weights far apart (the tile path stores mantissa +
+ * exponent and sums in exponent bands of 100 binary orders, each in units of its largest power of two, scaled back in
+ * float64). */
 int ast_project2d(const ast_project2d_params *p, const double *pos, const double *h,
                   const double *const *prop, double *out, void *workspace, size_t workspace_bytes,
                   void *stream, ast_project2d_stats *stats);
