@@ -119,6 +119,38 @@ __device__ __forceinline__ float shape_half_outer(float s)
     const float a1 = __saturatef(fmaf(fast_sqrt(s), -0.5f, 1.0f));
     return a1 * a1 * a1;
 }
+
+// The same three forms on a PAIR of pixels, for the packed float32 pipes of sm_100 (FFMA2 / FMUL2 / FADD2 through
+// __ffma2_rn / __fmul2_rn / __fadd2_rn).  Each component of a packed rn operation rounds exactly like its scalar twin and the
+// expression trees are those of the scalar forms, so every value is bit-identical to them.  There is no packed square root
+// and no packed saturate or minimum: MUFU.SQRT, FFMA.SAT and FMNMX stay scalar.  Shapes other than the cubic spline go
+// through the scalar form component by component.
+__device__ __forceinline__ float2 f2(float v) { return make_float2(v, v); }
+__device__ __forceinline__ float2 fast_sqrt2(float2 s) { return make_float2(fast_sqrt(s.x), fast_sqrt(s.y)); }
+__device__ __forceinline__ float2 half_outer_of_q2(float2 q)          // sat(1 - q/2)^3
+{
+    const float2 a1 = make_float2(__saturatef(fmaf(q.x, -0.5f, 1.0f)), __saturatef(fmaf(q.y, -0.5f, 1.0f)));
+    return __fmul2_rn(__fmul2_rn(a1, a1), a1);
+}
+template <int SHAPE>
+__device__ __forceinline__ float2 shape_half_full2(float2 s, const ShapeTab &tab)
+{
+    if (SHAPE == SHAPE_CUBIC) {
+        const float2 q = fast_sqrt2(s);
+        const float2 p = __ffma2_rn(s, __ffma2_rn(f2(0.375f), q, f2(-0.75f)), f2(0.5f));
+        const float2 o = half_outer_of_q2(q);
+        return make_float2(fminf(p.x, o.x), fminf(p.y, o.y));
+    }
+    return make_float2(shape_half_full<SHAPE>(s.x, tab), shape_half_full<SHAPE>(s.y, tab));
+}
+__device__ __forceinline__ float2 shape_half_inner2(float2 s)
+{
+    return __ffma2_rn(s, __ffma2_rn(f2(0.375f), fast_sqrt2(s), f2(-0.75f)), f2(0.5f));
+}
+__device__ __forceinline__ float2 shape_half_outer2(float2 s)
+{
+    return half_outer_of_q2(fast_sqrt2(s));
+}
 #endif
 
 }  // namespace ast

@@ -705,6 +705,11 @@ __global__ void __launch_bounds__(256) pair_record_kernel(Acc a, int64_t n, uint
 // 1 - 3/2 q^2 + 3/4 q^3 of _kernels.pyx:17, the second the outer branch 1/4 (2-q)^3 of :19; inner - outer = -(1-q)^3/2
 // changes sign exactly at q = 1, so the minimum selects the right branch and is 0 beyond q = 2), with the weights
 // doubled at staging time.  Sparse batches (fewer than kRowColMinHits hits) take the classic per-lane coordinates.
+// The quad is evaluated as two pixel pairs, one per column, with the packed float32 forms of ast_math.h (bit-identical to
+// the scalar ones): per pixel of the full list the SASS is 1/2 FADD2, MUFU.SQRT, FFMA.SAT, 1 FFMA2 and 1 FMUL2 of shape,
+// FMNMX and NP/2 FFMA2, i.e. 6 instructions for NP = 1 (7 with the slot loads and the loop control), 3 in the inner-only
+// and 4 in the outer-annulus list.  This saves issue slots, not FMA-pipe time: a packed instruction holds the FMA pipe for
+// two cycles, so a full-list pixel still costs ~7 FMA-pipe cycles next to the 8 XU cycles of its warp-wide MUFU.SQRT.
 constexpr int kRowColMinHits = 8;
 struct __align__(16) RowColSlot {
     float4 ax[2];        // squared x-distance (in h) to the 8 pixel columns of the sub-tile
@@ -736,12 +741,27 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
     RowColSlot *const slots = sS[warp];
     // classic view of the same storage: {ux*sx, uy*sy, sx, sy} in ax[0], {c0, c1} in the first half of ax[1]
 
-    float acc[NP][NPIX];
+    // float32 sums per pixel pair: acc[k][ix] = {pixel (xl + ix, yl), pixel (xl + ix, yl + 1)}, the two rows of one column,
+    // whose row values sit side by side in byc and whose column value is a broadcast operand of FADD2
+    float2 acc[NP][PX];
     double acc64[NP][NPIX];
 #pragma unroll
-    for (int k = 0; k < NP; ++k)
+    for (int k = 0; k < NP; ++k) {
 #pragma unroll
-        for (int j = 0; j < NPIX; ++j) { acc[k][j] = 0.f; acc64[k][j] = 0.0; }
+        for (int ix = 0; ix < PX; ++ix) acc[k][ix] = f2(0.f);
+#pragma unroll
+        for (int j = 0; j < NPIX; ++j) acc64[k][j] = 0.0;
+    }
+    // one staged entry of a dense batch: the lane's two column values, its two row values and the weights
+    auto eval_slot = [&](int e, auto shape2) {
+        const float2 ax2 = reinterpret_cast<const float2 *>(slots[e].ax)[lane >> 3];
+        const float4 bc = slots[e].byc[lane & 7];
+        const float2 by = make_float2(bc.x, bc.y);
+        const float2 f0 = shape2(__fadd2_rn(by, f2(ax2.x))), f1 = shape2(__fadd2_rn(by, f2(ax2.y)));
+        acc[0][0] = __ffma2_rn(f2(bc.z), f0, acc[0][0]); acc[0][1] = __ffma2_rn(f2(bc.z), f1, acc[0][1]);
+        if (NP > 1) { acc[NP - 1][0] = __ffma2_rn(f2(bc.w), f0, acc[NP - 1][0]); acc[NP - 1][1] = __ffma2_rn(f2(bc.w), f1, acc[NP - 1][1]); }
+    };
+    const auto full2 = [&](float2 s) { return shape_half_full2<SHAPE>(s, a.tab); };
 
     int since_fold = 0;
     for (uint32_t base = w_first; base < total; base += w_step) {
@@ -788,44 +808,15 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
                 }
             }
             __syncwarp();
-            for (int e = 0; e < nf; ++e) {
-                const float2 ax2 = reinterpret_cast<const float2 *>(slots[e].ax)[lane >> 3];
-                const float4 bc = slots[e].byc[lane & 7];
-                const float s00 = ax2.x + bc.x, s01 = ax2.x + bc.y, s10 = ax2.y + bc.x, s11 = ax2.y + bc.y;
-                const float f00 = shape_half_full<SHAPE>(s00, a.tab), f01 = shape_half_full<SHAPE>(s01, a.tab);
-                const float f10 = shape_half_full<SHAPE>(s10, a.tab), f11 = shape_half_full<SHAPE>(s11, a.tab);
-                acc[0][0] = fmaf(bc.z, f00, acc[0][0]); acc[0][1] = fmaf(bc.z, f01, acc[0][1]);
-                acc[0][2] = fmaf(bc.z, f10, acc[0][2]); acc[0][3] = fmaf(bc.z, f11, acc[0][3]);
-                if (NP > 1) {
-                    acc[NP - 1][0] = fmaf(bc.w, f00, acc[NP - 1][0]); acc[NP - 1][1] = fmaf(bc.w, f01, acc[NP - 1][1]);
-                    acc[NP - 1][2] = fmaf(bc.w, f10, acc[NP - 1][2]); acc[NP - 1][3] = fmaf(bc.w, f11, acc[NP - 1][3]);
-                }
-            }
+            // unrolled by 4: one entry per iteration spends ~7 of its ~33 instructions on the loop control and the slot address
+#pragma unroll 4
+            for (int e = 0; e < nf; ++e) eval_slot(e, full2);
             if (SHAPE == SHAPE_CUBIC) {
-                for (int e = nf; e < nf + ni; ++e) {            // every pixel of the sub-tile has q < 1: f/2 = 1/2 + s (3q/8 - 3/4)
-                    const float2 ax2 = reinterpret_cast<const float2 *>(slots[e].ax)[lane >> 3];
-                    const float4 bc = slots[e].byc[lane & 7];
-                    const float f00 = shape_half_inner(ax2.x + bc.x), f01 = shape_half_inner(ax2.x + bc.y);
-                    const float f10 = shape_half_inner(ax2.y + bc.x), f11 = shape_half_inner(ax2.y + bc.y);
-                    acc[0][0] = fmaf(bc.z, f00, acc[0][0]); acc[0][1] = fmaf(bc.z, f01, acc[0][1]);
-                    acc[0][2] = fmaf(bc.z, f10, acc[0][2]); acc[0][3] = fmaf(bc.z, f11, acc[0][3]);
-                    if (NP > 1) {
-                        acc[NP - 1][0] = fmaf(bc.w, f00, acc[NP - 1][0]); acc[NP - 1][1] = fmaf(bc.w, f01, acc[NP - 1][1]);
-                        acc[NP - 1][2] = fmaf(bc.w, f10, acc[NP - 1][2]); acc[NP - 1][3] = fmaf(bc.w, f11, acc[NP - 1][3]);
-                    }
-                }
-                for (int e = 32 - no; e < 32; ++e) {
-                    const float2 ax2 = reinterpret_cast<const float2 *>(slots[e].ax)[lane >> 3];
-                    const float4 bc = slots[e].byc[lane & 7];
-                    const float f00 = shape_half_outer(ax2.x + bc.x), f01 = shape_half_outer(ax2.x + bc.y);
-                    const float f10 = shape_half_outer(ax2.y + bc.x), f11 = shape_half_outer(ax2.y + bc.y);
-                    acc[0][0] = fmaf(bc.z, f00, acc[0][0]); acc[0][1] = fmaf(bc.z, f01, acc[0][1]);
-                    acc[0][2] = fmaf(bc.z, f10, acc[0][2]); acc[0][3] = fmaf(bc.z, f11, acc[0][3]);
-                    if (NP > 1) {
-                        acc[NP - 1][0] = fmaf(bc.w, f00, acc[NP - 1][0]); acc[NP - 1][1] = fmaf(bc.w, f01, acc[NP - 1][1]);
-                        acc[NP - 1][2] = fmaf(bc.w, f10, acc[NP - 1][2]); acc[NP - 1][3] = fmaf(bc.w, f11, acc[NP - 1][3]);
-                    }
-                }
+                // every pixel has q < 1: f/2 = 1/2 + s (3q/8 - 3/4)
+#pragma unroll 4
+                for (int e = nf; e < nf + ni; ++e) eval_slot(e, [](float2 s) { return shape_half_inner2(s); });
+#pragma unroll 4
+                for (int e = 32 - no; e < 32; ++e) eval_slot(e, [](float2 s) { return shape_half_outer2(s); });
             }
         } else {
             if (hit) {
@@ -843,14 +834,14 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
                 for (int i = 0; i < PX; ++i) { const float t = fmaf(-xf[i], q.z, q.x); ax2[i] = t * t; }
 #pragma unroll
                 for (int i = 0; i < PY; ++i) { const float t = fmaf(-yf[i], q.w, q.y); by2[i] = t * t; }
+                // scalar on purpose: ax2 + by2 of two products in registers is contracted to an FFMA here, which a packed
+                // FADD2 would not reproduce bit for bit
 #pragma unroll
-                for (int ix = 0; ix < PX; ++ix)
-#pragma unroll
-                    for (int iy = 0; iy < PY; ++iy) {
-                        const float f = shape_half_full<SHAPE>(ax2[ix] + by2[iy], a.tab);
-                        acc[0][ix * PY + iy] = fmaf(c.x, f, acc[0][ix * PY + iy]);
-                        if (NP > 1) acc[NP - 1][ix * PY + iy] = fmaf(c.y, f, acc[NP - 1][ix * PY + iy]);
-                    }
+                for (int ix = 0; ix < PX; ++ix) {
+                    const float f0 = shape_half_full<SHAPE>(ax2[ix] + by2[0], a.tab), f1 = shape_half_full<SHAPE>(ax2[ix] + by2[1], a.tab);
+                    acc[0][ix].x = fmaf(c.x, f0, acc[0][ix].x); acc[0][ix].y = fmaf(c.x, f1, acc[0][ix].y);
+                    if (NP > 1) { acc[NP - 1][ix].x = fmaf(c.y, f0, acc[NP - 1][ix].x); acc[NP - 1][ix].y = fmaf(c.y, f1, acc[NP - 1][ix].y); }
+                }
             }
         }
         __syncwarp();
@@ -860,7 +851,11 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
 #pragma unroll
             for (int k = 0; k < NP; ++k)
 #pragma unroll
-                for (int jj = 0; jj < NPIX; ++jj) { acc64[k][jj] += (double)acc[k][jj]; acc[k][jj] = 0.f; }
+                for (int ix = 0; ix < PX; ++ix) {
+                    acc64[k][ix * PY] += (double)acc[k][ix].x;
+                    acc64[k][ix * PY + 1] += (double)acc[k][ix].y;
+                    acc[k][ix] = f2(0.f);
+                }
         }
     }
     // the sums are in units of 2^etop_k: two exact power-of-two factors (etop_k spans -1073 .. 1024, one factor could overflow)
@@ -882,7 +877,7 @@ __global__ void __launch_bounds__(256, 3) rowcol_accum_kernel(Acc a)
 #pragma unroll
             for (int k = 0; k < NP; ++k) {
                 double *o = a.out + k * a.map_stride + (size_t)xi * a.ny + yi;
-                const double v = (acc64[k][ix * PY + iy] + (double)acc[k][ix * PY + iy]) * sc1[k] * sc2[k];
+                const double v = (acc64[k][ix * PY + iy] + (double)(iy ? acc[k][ix].y : acc[k][ix].x)) * sc1[k] * sc2[k];
                 if (w.atomic_out) atomicAdd(o, v); else *o += v;
             }
         }
