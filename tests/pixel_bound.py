@@ -23,8 +23,13 @@ Sum: ~1.2e-5, below tau with a factor 2.6 to spare.  The direct-deposit paths (f
 only) are well inside the same bound.  Weights flushed to zero because they lie far below the largest weight of the call
 are errors of up to env itself, i.e. tau^-1 = 32768 times the bound.
 
-Outside this bound, on purpose: scenes that force sub-half-pixel h through the tile path (the q error grows as 1/h there),
-and AST_KERNEL_TABLE, whose table interpolation error is a separate, separately tested matter.
+The bound holds for tabulated kernels (AST_KERNEL_TABLE) too, when the kernel is continuous and zero at q = 2: the table
+has 8192 intervals on q in [0, 2], so linear interpolation is off by at most dq^2 max|f''| / 8 ~ 2e-8 of f(0), and the
+float32 table entries add 2^-24.  The kernel callable can be passed in place of a name (W(0, h) = kernel(0, h)).
+
+Outside this bound, on purpose: scenes that force h below half the largest cell side through the tile or brick path (the
+q error grows as cell / h there), and tables of kernels that are discontinuous at q = 2 (a truncated Gaussian, say),
+whose interpolation error at the jump is of the order of the jump itself.
 """
 import numpy as np
 
@@ -37,11 +42,16 @@ _PLANE = {0: (1, 2), 1: (0, 2), 2: (0, 1)}
 
 
 def _peaks(prop, h, kernel):
-    """|prop| W(0, h) as (P, N), and the particles that have a support at all"""
+    """|prop| W(0, h) as (P, N), and the particles that have a support at all; kernel: a built-in name or id, or a
+    callable kernel_func(r, h)"""
     ok = (h > 0) & np.isfinite(2.0 * h)
     w0 = np.zeros(h.shape)
     if ok.any():
-        w0[ok] = oracle.kernel_eval(kernel, np.zeros(int(ok.sum())), h[ok])
+        hk = np.ascontiguousarray(h[ok], dtype=np.float64)
+        if callable(kernel):
+            w0[ok] = np.asarray(kernel(np.zeros(hk.size), hk), dtype=np.float64)
+        else:
+            w0[ok] = oracle.kernel_eval(kernel, np.zeros(hk.size), hk)
     return np.abs(prop) * w0, ok
 
 
