@@ -39,7 +39,8 @@ class Grid3DParams(C.Structure):
                 ("lo", C.c_double * 3), ("hi", C.c_double * 3), ("box", C.c_double * 3),
                 ("small_max_vox", C.c_int64), ("huge_min_bricks", C.c_int64),
                 ("pair_capacity", C.c_int64), ("huge_capacity", C.c_int64),
-                ("kernel_table", C.c_void_p), ("kernel_table_n", C.c_int32), ("kernel_dim", C.c_int32)]
+                ("kernel_table", C.c_void_p), ("kernel_table_n", C.c_int32), ("kernel_dim", C.c_int32),
+                ("x_begin", C.c_int32), ("x_end", C.c_int32)]
 
 
 class KnnParams(C.Structure):
@@ -66,6 +67,13 @@ class SlabRouteParams(C.Structure):
                 ("length", C.c_double), ("w", C.c_double), ("bounds", C.c_double * (ROUTE_MAX_WORLD + 1))]
 
 
+class GridRouteParams(C.Structure):
+    _fields_ = [("n", C.c_int64), ("world", C.c_int32), ("periodic", C.c_int32),
+                ("nx", C.c_int32), ("ny", C.c_int32), ("nz", C.c_int32), ("reserved", C.c_int32),
+                ("lo", C.c_double * 3), ("hi", C.c_double * 3), ("box", C.c_double * 3),
+                ("edges", C.c_int32 * (ROUTE_MAX_WORLD + 1))]
+
+
 class WorkspaceError(RuntimeError):
     """AST_EWORKSPACE: a capacity or the workspace was too small (message says what is needed)."""
 
@@ -77,6 +85,7 @@ EXPORTS = ["ast_project2d_workspace_bytes", "ast_project2d", "ast_bin2d", "ast_c
            "ast_sort_workspace_bytes", "ast_radix_sort_u64", "ast_grid3d_workspace_bytes", "ast_grid3d", "ast_bin3d",
            "ast_knn_workspace_bytes", "ast_knn_h", "ast_knn_query", "ast_match_ids_workspace_bytes", "ast_match_ids", "ast_gather_rows", "ast_table_interp",
            "ast_slab_route_workspace_bytes", "ast_slab_route_count", "ast_slab_route_write",
+           "ast_grid_route_workspace_bytes", "ast_grid_route_count", "ast_grid_route_write",
            "ast_last_error", "ast_abi_version", "ast_tile_size",
            "ast_device_sm_count"]
 

@@ -187,8 +187,14 @@ struct Bin3 {
     int cls;
 };
 
+// x window of a grid: planes [x0, x0 + n) of the whole grid's x axis.  The axes stay the whole grid's, so every sample
+// point and every contributor range is the whole grid's value; bboxes and bricks are numbered from x0.
+struct Win1 {
+    int x0, n;
+};
+
 template <int BRICK>
-AST_HD Bin3 classify3(const Axis1 *ax /* [3] */, const double *p /* [3] */, double h, double R2, int64_t small_max_vox,
+AST_HD Bin3 classify3(const Axis1 *ax /* [3] */, Win1 w, const double *p /* [3] */, double h, double R2, int64_t small_max_vox,
                       int64_t huge_min_bricks)
 {
     Bin3 b;
@@ -197,6 +203,9 @@ AST_HD Bin3 classify3(const Axis1 *ax /* [3] */, const double *p /* [3] */, doub
     int lo[3], hi[3];
     for (int c = 0; c < 3; ++c)
         if (!range1(ax[c], p[c], h, R2, lo[c], hi[c])) return b;
+    lo[0] = (lo[0] > w.x0 ? lo[0] : w.x0) - w.x0;                      // clip the whole grid's x range to the window
+    hi[0] = (hi[0] < w.x0 + w.n - 1 ? hi[0] : w.x0 + w.n - 1) - w.x0;
+    if (lo[0] > hi[0]) return b;
     int64_t vol = 1, nb = 1;
     for (int c = 0; c < 3; ++c) {
         b.lo[c] = lo[c]; b.hi[c] = hi[c];
@@ -211,15 +220,16 @@ AST_HD Bin3 classify3(const Axis1 *ax /* [3] */, const double *p /* [3] */, doub
     return b;
 }
 
-// bricks in emit order (bx, by, bz ascending) that hold at least one voxel with (dx^2 + dy^2) + dz^2 < R2
+// bricks in emit order (bx, by, bz ascending) that hold at least one voxel with (dx^2 + dy^2) + dz^2 < R2; b from classify3
+// on the window that starts at plane x0
 template <int BRICK, class F>
-AST_HD int for_each_brick3(const Axis1 *ax, const double *p, double R2, const Bin3 &b, int nby, int nbz, F &&f)
+AST_HD int for_each_brick3(const Axis1 *ax, int x0, const double *p, double R2, const Bin3 &b, int nby, int nbz, F &&f)
 {
     int cnt = 0;
     for (int bx = b.b0[0]; bx <= b.b1[0]; ++bx) {
         int xa = bx * BRICK > b.lo[0] ? bx * BRICK : b.lo[0];
         int xb = bx * BRICK + BRICK - 1 < b.hi[0] ? bx * BRICK + BRICK - 1 : b.hi[0];
-        double mdx = min_dist2(ax[0], p[0], xa, xb);
+        double mdx = min_dist2(ax[0], p[0], x0 + xa, x0 + xb);
         for (int by = b.b0[1]; by <= b.b1[1]; ++by) {
             int ya = by * BRICK > b.lo[1] ? by * BRICK : b.lo[1];
             int yb = by * BRICK + BRICK - 1 < b.hi[1] ? by * BRICK + BRICK - 1 : b.hi[1];

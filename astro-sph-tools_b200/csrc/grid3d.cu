@@ -33,8 +33,9 @@ struct P3 {
     double *out;
     int64_t n;
     int kernel_id, shape;
-    Axis1 ax[3];
-    int nb[3];                       // bricks per axis
+    Axis1 ax[3];                     // the whole grid's axes
+    Win1 win;                        // the planes this call computes (ast_grid3d_params x_begin / x_end)
+    int nb[3];                       // bricks per axis (x: of the window)
     int n_img, img_shift;
     double box[3];                   // periodic image m = 9*(ia+1) + 3*(ib+1) + (ic+1), shift = (ia,ib,ic) * box
     ShapeTab tab;
@@ -145,7 +146,7 @@ __device__ __forceinline__ void deposit_small3(const P3 &p, const Bin3 &b, const
     const double inv_h2 = 1.0 / (h * h);
     const size_t ny = p.ax[1].n, nz = p.ax[2].n;
     for (int xi = b.lo[0]; xi <= b.hi[0]; ++xi) {
-        const double dx2 = dist2(p.ax[0], q[0], xi);
+        const double dx2 = dist2(p.ax[0], q[0], p.win.x0 + xi);
         for (int yi = b.lo[1]; yi <= b.hi[1]; ++yi) {
             const double dxy = AST_DADD(dx2, dist2(p.ax[1], q[1], yi));
             double *row = p.out + ((size_t)xi * ny + yi) * nz;
@@ -157,8 +158,9 @@ __device__ __forceinline__ void deposit_small3(const P3 &p, const Bin3 &b, const
     }
 }
 
+// (at least 2 blocks of 256 per SM: without that bound ptxas capped some instantiations at 80 registers and spilled)
 template <int SHAPE, bool DEPOSIT>
-__global__ void __launch_bounds__(kBin3Threads) bin3_kernel(P3 p, Rec3 *__restrict__ rec, uint64_t *__restrict__ block_pairs,
+__global__ void __launch_bounds__(kBin3Threads, 2) bin3_kernel(P3 p, Rec3 *__restrict__ rec, uint64_t *__restrict__ block_pairs,
                                                             uint64_t *__restrict__ block_huge)
 {
     __shared__ uint32_t red[34];
@@ -182,11 +184,11 @@ __global__ void __launch_bounds__(kBin3Threads) bin3_kernel(P3 p, Rec3 *__restri
                     q[2] = AST_DADD(x0[2], p.n_img == 1 ? 0.0 : (double)(ic - 1) * p.box[2]);
                     if (!may_touch(p.ax[2], q[2], h2)) continue;
                     const int m = 9 * ia + 3 * ib + ic;
-                    Bin3 b = classify3<BRICK>(p.ax, q, h, R2, p.small_max_vox, p.huge_min_bricks);
+                    Bin3 b = classify3<BRICK>(p.ax, p.win, q, h, R2, p.small_max_vox, p.huge_min_bricks);
                     if (b.cls == CLS_SMALL) {
                         if (DEPOSIT) deposit_small3<SHAPE>(p, b, q, h, R2, p.prop[i] * norm3(p, h));
                     } else if (b.cls == CLS_TILED) {
-                        npairs += (uint32_t)for_each_brick3<BRICK>(p.ax, q, R2, b, p.nb[1], p.nb[2], [](uint32_t) {});
+                        npairs += (uint32_t)for_each_brick3<BRICK>(p.ax, p.win.x0, q, R2, b, p.nb[1], p.nb[2], [](uint32_t) {});
                         mask |= 1ull << m;
                         need_rec = true;
                     } else if (b.cls == CLS_HUGE) {
@@ -243,10 +245,10 @@ __global__ void __launch_bounds__(kBin3Threads, 3) emit3_kernel(P3 p, const uint
     for (int m = 0; m < p.n_img; ++m) {
         if (!((mask >> m) & 0x8000001ull)) continue;                       // image m has neither pairs nor a large-h entry
         const double q[3] = { AST_DADD(x0[0], image_shift3(p.n_img, p.box, m, 0)), AST_DADD(x0[1], image_shift3(p.n_img, p.box, m, 1)), AST_DADD(x0[2], image_shift3(p.n_img, p.box, m, 2)) };
-        Bin3 b = classify3<BRICK>(p.ax, q, h, R2, p.small_max_vox, p.huge_min_bricks);
+        Bin3 b = classify3<BRICK>(p.ax, p.win, q, h, R2, p.small_max_vox, p.huge_min_bricks);
         if (b.cls == CLS_TILED) {
             if (!any_pairs) continue;
-            for_each_brick3<BRICK>(p.ax, q, R2, b, p.nb[1], p.nb[2], [&](uint32_t key) {
+            for_each_brick3<BRICK>(p.ax, p.win.x0, q, R2, b, p.nb[1], p.nb[2], [&](uint32_t key) {
                 if (g >= w0 && g < w1)
                     pairs[g - w0] = ((uint64_t)((key << p.img_shift) | (uint32_t)m) << 32) | (uint64_t)(uint32_t)i;
                 ++g;
@@ -283,7 +285,7 @@ __global__ void __launch_bounds__(256) huge_bricks_kernel(P3 p, const uint64_t *
     const double h = p.h[i], R2 = radius2(h);
     const double q[3] = { AST_DADD(p.pos[3 * i], image_shift3(p.n_img, p.box, m, 0)), AST_DADD(p.pos[3 * i + 1], image_shift3(p.n_img, p.box, m, 1)),
                           AST_DADD(p.pos[3 * i + 2], image_shift3(p.n_img, p.box, m, 2)) };
-    const Bin3 b = classify3<BRICK>(p.ax, q, h, R2, p.small_max_vox, p.huge_min_bricks);
+    const Bin3 b = classify3<BRICK>(p.ax, p.win, q, h, R2, p.small_max_vox, p.huge_min_bricks);
     const int ny_b = b.b1[1] - b.b0[1] + 1, nz_b = b.b1[2] - b.b0[2] + 1;
     const int64_t nt = (int64_t)(b.b1[0] - b.b0[0] + 1) * ny_b * nz_b;
     uint32_t cnt = 0;
@@ -300,7 +302,8 @@ __global__ void __launch_bounds__(256) huge_bricks_kernel(P3 p, const uint64_t *
             for (int c = 0; c < 3; ++c) {
                 const int a0 = bc[c] * BRICK > b.lo[c] ? bc[c] * BRICK : b.lo[c];
                 const int a1 = bc[c] * BRICK + BRICK - 1 < b.hi[c] ? bc[c] * BRICK + BRICK - 1 : b.hi[c];
-                md[c] = min_dist2(p.ax[c], q[c], a0, a1);
+                const int off = c == 0 ? p.win.x0 : 0;
+                md[c] = min_dist2(p.ax[c], q[c], off + a0, off + a1);
             }
             in = AST_DADD(AST_DADD(md[0], md[1]), md[2]) < R2;
             key = (uint32_t)((bx * p.nb[1] + by) * p.nb[2] + bz);
@@ -336,7 +339,8 @@ struct Acc3 {
     const Rec3 *rec;
     double *out;
     double lo[3], d[3], inv_d[3];
-    int n[3], nb[3], img_shift, n_img;
+    int n[3], nb[3], img_shift, n_img;   // n[0], nb[0]: planes and bricks of the window
+    double x0;                           // first plane of the window in the whole grid
     double box[3];
     ShapeTab tab;
     const uint32_t *seg_off;     // work items over the brick lists (work_items.cuh); ntiles = number of bricks
@@ -394,7 +398,7 @@ __global__ void __launch_bounds__(kAcc3Threads) brick_accum_kernel(Acc3 a)
             const uint64_t e = a.sorted[beg + j];
             const uint32_t idx = (uint32_t)e, m = ((uint32_t)(e >> 32)) & ((1u << a.img_shift) - 1u);
             const Rec3 r = a.rec[idx];
-            const float fx = (float)((r.x + image_shift3(a.n_img, a.box, (int)m, 0) - a.lo[0]) * a.inv_d[0] - (double)X0);
+            const float fx = (float)((r.x + image_shift3(a.n_img, a.box, (int)m, 0) - a.lo[0]) * a.inv_d[0] - (double)X0 - a.x0);
             const float fy = (float)((r.y + image_shift3(a.n_img, a.box, (int)m, 1) - a.lo[1]) * a.inv_d[1] - (double)Y0);
             const float fz = (float)((r.z + image_shift3(a.n_img, a.box, (int)m, 2) - a.lo[2]) * a.inv_d[2] - (double)Z0);
             const float sx = d0 * r.inv_h, sy = d1 * r.inv_h, sz = d2 * r.inv_h;
@@ -522,7 +526,7 @@ __global__ void bbox_cls3_kernel(P3 p, int32_t *__restrict__ bbox, uint8_t *__re
     const double h = p.h[i], R2 = radius2(h);
     for (int m = 0; m < p.n_img; ++m) {
         const double q[3] = { AST_DADD(x0[0], image_shift3(p.n_img, p.box, m, 0)), AST_DADD(x0[1], image_shift3(p.n_img, p.box, m, 1)), AST_DADD(x0[2], image_shift3(p.n_img, p.box, m, 2)) };
-        Bin3 b = classify3<BRICK>(p.ax, q, h, R2, p.small_max_vox, p.huge_min_bricks);
+        Bin3 b = classify3<BRICK>(p.ax, p.win, q, h, R2, p.small_max_vox, p.huge_min_bricks);
         const int64_t j = (int64_t)m * p.n + i;
         if (bbox)
             for (int c = 0; c < 3; ++c) { bbox[6 * j + 2 * c] = b.lo[c]; bbox[6 * j + 2 * c + 1] = b.hi[c]; }
@@ -548,12 +552,23 @@ struct Layout3 {
     size_t bytes;
 };
 
+// the planes a call computes: [x_begin, x_end), or the whole grid for 0, 0 (checked by validate3)
+static Win1 window3(const ast_grid3d_params *p)
+{
+    Win1 w;
+    w.x0 = p->x_end > 0 ? p->x_begin : 0;
+    w.n = p->x_end > 0 ? p->x_end - p->x_begin : p->nx;
+    return w;
+}
+
 static int validate3(const ast_grid3d_params *p)
 {
     AST_REQUIRE(p != nullptr, "params is null");
     AST_REQUIRE(p->n >= 0 && p->n < (int64_t)0xffffffffll, "n out of range");
     AST_REQUIRE(p->nx > 0 && p->ny > 0 && p->nz > 0, "grid size must be positive");
-    const int64_t nbr = (int64_t)((p->nx + BRICK - 1) / BRICK) * ((p->ny + BRICK - 1) / BRICK) * ((p->nz + BRICK - 1) / BRICK);
+    AST_REQUIRE((p->x_begin == 0 && p->x_end == 0) || (p->x_begin >= 0 && p->x_begin < p->x_end && p->x_end <= p->nx),
+                "x window [%d, %d) is not inside [0, nx = %d) (0, 0 = the whole grid)", p->x_begin, p->x_end, p->nx);
+    const int64_t nbr = (int64_t)((window3(p).n + BRICK - 1) / BRICK) * ((p->ny + BRICK - 1) / BRICK) * ((p->nz + BRICK - 1) / BRICK);
     AST_REQUIRE(nbr < (1ll << 26), "grid too large (more than 2^26 bricks)");
     AST_REQUIRE(kernel_valid(p->kernel_id), "unknown kernel id %d", p->kernel_id);
     if (p->kernel_id == AST_KERNEL_TABLE)
@@ -572,7 +587,7 @@ static Layout3 layout3(const ast_grid3d_params *p, void *ws)
     Layout3 L;
     L.nb = (p->n + kBin3Threads - 1) / kBin3Threads;
     if (L.nb < 1) L.nb = 1;
-    L.nbricks = (int64_t)((p->nx + BRICK - 1) / BRICK) * ((p->ny + BRICK - 1) / BRICK) * ((p->nz + BRICK - 1) / BRICK);
+    L.nbricks = (int64_t)((window3(p).n + BRICK - 1) / BRICK) * ((p->ny + BRICK - 1) / BRICK) * ((p->nz + BRICK - 1) / BRICK);
     L.pair_cap = p->pair_capacity > 0 ? p->pair_capacity : 1;
     L.huge_cap = p->huge_capacity > 0 ? p->huge_capacity : 1;
     Carver c(ws);
@@ -621,9 +636,10 @@ static P3 make_p3(const ast_grid3d_params *p, const double *pos, const double *h
     a.tab.n = p->kernel_table_n;
     a.tab.scale = 0.5f * (float)p->kernel_table_n;
     const int n3[3] = { p->nx, p->ny, p->nz };
+    a.win = window3(p);
     for (int c = 0; c < 3; ++c) {
         a.ax[c] = make_axis(p->lo[c], p->hi[c], n3[c]);
-        a.nb[c] = (n3[c] + BRICK - 1) / BRICK;
+        a.nb[c] = ((c == 0 ? a.win.n : n3[c]) + BRICK - 1) / BRICK;
     }
     const bool per = (p->flags & AST_FLAG_PERIODIC) != 0;
     a.n_img = per ? 27 : 1;
@@ -672,12 +688,14 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
         OrderGrid og;
         memset(&og, 0, sizeof og);
         og.dims = 3;
-        const int n3[3] = { p->nx, p->ny, p->nz };
+        const Win1 w = window3(p);
+        const int n3[3] = { p->nx, p->ny, p->nz }, nw[3] = { w.n, p->ny, p->nz };
         for (int k = 0; k < 3; ++k) {
+            const double d = (p->hi[k] - p->lo[k]) / n3[k];
             og.col[k] = k;
-            og.lo[k] = p->lo[k];
-            og.inv_cell[k] = 1.0 / ((p->hi[k] - p->lo[k]) / n3[k] * BRICK);
-            og.n[k] = (n3[k] + BRICK - 1) / BRICK;
+            og.lo[k] = k == 0 ? p->lo[k] + (double)w.x0 * d : p->lo[k];
+            og.inv_cell[k] = 1.0 / (d * BRICK);
+            og.n[k] = (nw[k] + BRICK - 1) / BRICK;
         }
         int done = 0, nl = 0;
         const double *props1[1] = { prop };
@@ -688,7 +706,7 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
     }
     P3 a = make_p3(p, pos, h, prop, out);
     a.pcount = L.pcount; a.pmask = L.pmask; a.wexp = L.wexp;
-    const size_t nvox = (size_t)p->nx * p->ny * p->nz;
+    const size_t nvox = (size_t)a.win.n * p->ny * p->nz;
     if (!(p->flags & AST_FLAG_ACCUMULATE)) AST_CUDA_TRY(cudaMemsetAsync(out, 0, sizeof(double) * nvox, s));
     AST_CUDA_TRY(cudaMemsetAsync(L.block_pairs, 0, sizeof(uint64_t) * (L.nb + 1), s));
     AST_CUDA_TRY(cudaMemsetAsync(L.block_huge, 0, sizeof(uint64_t) * (L.nb + 1), s));
@@ -740,6 +758,8 @@ extern "C" int ast_grid3d(const ast_grid3d_params *p, const double *pos, const d
         for (int k = 0; k < 3; ++k) {
             c.lo[k] = a.ax[k].vmin; c.d[k] = a.ax[k].d; c.inv_d[k] = a.ax[k].inv_d; c.n[k] = a.ax[k].n; c.nb[k] = a.nb[k];
         }
+        c.n[0] = a.win.n;
+        c.x0 = (double)a.win.x0;
         c.img_shift = a.img_shift;
         c.n_img = a.n_img;
         c.tab = a.tab;

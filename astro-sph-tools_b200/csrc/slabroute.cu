@@ -1,4 +1,5 @@
-// slabroute.cu -- packing kernel of the multi-GPU k-NN exchange (SURVEY 8(e): slabs along x + ghost zones).
+// slabroute.cu -- packing kernel of the multi-GPU exchanges along x-slabs: the k-NN exchange (SURVEY 8(e): slabs along x +
+// ghost zones) and the 3-D gridding exchange (each rank owns an x-slab of the grid).  One kernel, two destination policies.
 //
 // Every rank holds an arbitrary set of particles (the reference's per-rank read, io/EAGLE/_SnapshotEAGLE.py:120-130) and has
 // to send each of them to the rank that OWNS its slab and, as a ghost, to every rank whose slab lies within the ghost width
@@ -11,6 +12,8 @@
 // Send buffer layout: [owned -> rank 0 | owned -> rank 1 | ... | ghosts -> rank 0 | ghosts -> rank 1 | ...], inside each piece
 // ascending particle index (blocks, warps and lanes are walked in order), which is also what the torch version produces.
 // Two all-to-all calls (owned, then ghosts) then leave the receiver with [owned from all | ghosts from all] without a reorder.
+// Gridding has one kind: a particle goes to every rank whose planes its support reaches (GridRoute), rows (x, y, z, h, prop).
+#include "ast_geom.h"
 #include "common.cuh"
 #include "scan_sort.cuh"
 
@@ -18,82 +21,132 @@ namespace ast {
 
 constexpr int kRouteMaxWorld = 32;
 
-struct RouteArgs {
+// A destination policy R provides
+//   kKinds                    pieces of the send buffer per destination rank (kind-major: [kind 0 -> 0 | kind 0 -> 1 | ...])
+//   n, world                  local particles, ranks
+//   dests(i, m)               m[k] bit g: particle i goes to rank g as kind k (the count and the write pass call the same code)
+//   put(send, idx, row, i)    write particle i as send row `row`
+struct KnnRoute {
+    static constexpr int kKinds = 2;                 // 0 = owned, 1 = ghost
     const double *pos;            // (n, 3)
     const int64_t *owner;         // (n) owning rank of every particle (from the global histogram plan)
     int64_t n;
     int world, periodic, covers_all;
     double length, w;
     double b_lo[kRouteMaxWorld], b_hi[kRouteMaxWorld];
+
+    // bit g of the result: the particle goes to rank g as a ghost
+    __device__ __forceinline__ uint32_t ghosts(double x, int own) const
+    {
+        uint32_t m = 0;
+        for (int g = 0; g < world; ++g) {
+            if (g == own) continue;
+            double d;
+            if (periodic) {
+                double t = fmod(x - b_lo[g], length);
+                if (t < 0.0) t += length;
+                const double seg = b_hi[g] - b_lo[g];
+                d = t <= seg ? 0.0 : fmin(t - seg, length - t);
+            } else {
+                d = fmax(fmax(b_lo[g] - x, x - b_hi[g]), 0.0);
+            }
+            if (d <= w || covers_all) m |= 1u << g;
+        }
+        return m;
+    }
+    __device__ __forceinline__ void dests(int64_t i, uint32_t *m) const
+    {
+        int own = (int)owner[i];
+        if (own < 0 || own >= world) own = -1;                         // (never from _slab_plan; such a particle would be dropped)
+        m[0] = own >= 0 ? 1u << own : 0u;
+        m[1] = ghosts(pos[3 * i], own);
+    }
+    __device__ __forceinline__ void put(double *send, int64_t *src_index, int64_t row, int64_t i) const
+    {
+        send[3 * row] = pos[3 * i]; send[3 * row + 1] = pos[3 * i + 1]; send[3 * row + 2] = pos[3 * i + 2];
+        src_index[row] = i;
+    }
 };
 
-// bit g of the result: the particle goes to rank g as a ghost
-__device__ __forceinline__ uint32_t route_ghosts(const RouteArgs &a, double x, int own)
-{
-    uint32_t m = 0;
-    for (int g = 0; g < a.world; ++g) {
-        if (g == own) continue;
-        double d;
-        if (a.periodic) {
-            double t = fmod(x - a.b_lo[g], a.length);
-            if (t < 0.0) t += a.length;
-            const double seg = a.b_hi[g] - a.b_lo[g];
-            d = t <= seg ? 0.0 : fmin(t - seg, a.length - t);
-        } else {
-            d = fmax(fmax(a.b_lo[g] - x, x - a.b_hi[g]), 0.0);
-        }
-        if (d <= a.w || a.covers_all) m |= 1u << g;
-    }
-    return m;
-}
+// Rank g owns planes [e[g], e[g+1]) of the whole grid.  The ranges are range1 on the whole grid's axes and the image shifts
+// are bin3_kernel's, so a particle reaches a rank exactly when ast_grid3d with that rank's x window would deposit it.
+struct GridRoute {
+    static constexpr int kKinds = 1;
+    const double *pos, *h, *prop;
+    int64_t n;
+    int world, periodic;
+    Axis1 ax[3];
+    double box[3];
+    int e[kRouteMaxWorld + 1];
 
-// table[(kind * world + g) * nblocks + block], kind 0 = owned, 1 = ghost
-template <bool WRITE>
-__global__ void __launch_bounds__(256) slab_route_kernel(RouteArgs a, uint64_t *__restrict__ table, int64_t nblocks,
-                                                         double *__restrict__ send, int64_t *__restrict__ src_index)
+    __device__ __forceinline__ void dests(int64_t i, uint32_t *m) const
+    {
+        m[0] = 0u;
+        const double hh = h[i], R2 = radius2(hh);
+        const int nt = periodic ? 3 : 1;
+        int lo, up;
+        for (int c = 1; c < 3; ++c) {                                    // some image must reach the grid along y and along z
+            bool any = false;
+            for (int t = 0; t < nt && !any; ++t)
+                any = range1(ax[c], AST_DADD(pos[3 * i + c], periodic ? (double)(t - 1) * box[c] : 0.0), hh, R2, lo, up);
+            if (!any) return;
+        }
+        for (int t = 0; t < nt; ++t) {
+            if (!range1(ax[0], AST_DADD(pos[3 * i], periodic ? (double)(t - 1) * box[0] : 0.0), hh, R2, lo, up)) continue;
+            for (int g = 0; g < world; ++g)
+                if (e[g] < e[g + 1] && e[g] <= up && lo < e[g + 1]) m[0] |= 1u << g;
+        }
+    }
+    __device__ __forceinline__ void put(double *send, int64_t *, int64_t row, int64_t i) const
+    {
+        double *r = send + 5 * row;
+        r[0] = pos[3 * i]; r[1] = pos[3 * i + 1]; r[2] = pos[3 * i + 2]; r[3] = h[i]; r[4] = prop[i];
+    }
+};
+
+// table[(kind * world + g) * nblocks + block].  WRITE: a row at or beyond send_rows (the rows the caller allocated from the
+// counted total) is not written; it sets *overflow instead.
+template <class R, bool WRITE>
+__global__ void __launch_bounds__(256) slab_route_kernel(R a, uint64_t *__restrict__ table, int64_t nblocks, double *__restrict__ send,
+                                                         int64_t *__restrict__ src_index, int64_t send_rows, int *__restrict__ overflow)
 {
     __shared__ uint32_t wcount[2 * kRouteMaxWorld][8];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t i = (int64_t)blockIdx.x * 256 + tid;
-    const bool valid = i < a.n;
-    int own = -1;
-    uint32_t gm = 0;
-    double x = 0.0, y = 0.0, z = 0.0;
-    if (valid) {
-        x = a.pos[3 * i];
-        own = (int)a.owner[i];
-        if (own < 0 || own >= a.world) own = -1;                       // (never from _slab_plan; such a particle would be dropped)
-        gm = route_ghosts(a, x, own);
-        if (WRITE) { y = a.pos[3 * i + 1]; z = a.pos[3 * i + 2]; }
-    }
-    const unsigned lt = (1u << lane) - 1u;
-    for (int g = 0; g < a.world; ++g) {
-        const unsigned bo = __ballot_sync(0xffffffffu, own == g), bg = __ballot_sync(0xffffffffu, (gm >> g) & 1u);
-        if (lane == 0) { wcount[g][warp] = __popc(bo); wcount[a.world + g][warp] = __popc(bg); }
-    }
+    uint32_t m[R::kKinds];
+    for (int k = 0; k < R::kKinds; ++k) m[k] = 0u;
+    if (i < a.n) a.dests(i, m);
+    for (int k = 0; k < R::kKinds; ++k)
+        for (int g = 0; g < a.world; ++g) {
+            const unsigned b = __ballot_sync(0xffffffffu, (m[k] >> g) & 1u);
+            if (lane == 0) wcount[k * a.world + g][warp] = __popc(b);
+        }
     __syncthreads();
     if (!WRITE) {
-        if (tid < 2 * a.world) {
+        if (tid < R::kKinds * a.world) {
             uint32_t s = 0;
             for (int w = 0; w < 8; ++w) s += wcount[tid][w];
             table[(int64_t)tid * nblocks + blockIdx.x] = s;
         }
+        return;
     }
     // (all lanes stay to the end: the ballots below are full-warp)
-    for (int g = 0; WRITE && g < a.world; ++g) {
-        const bool is_own = own == g, is_ghost = (gm >> g) & 1u;
-        const unsigned bo = __ballot_sync(0xffffffffu, is_own), bg = __ballot_sync(0xffffffffu, is_ghost);
-        if (!is_own && !is_ghost) continue;
-        const int piece = is_own ? g : a.world + g;
-        uint32_t before = 0;
-        for (int w = 0; w < warp; ++w) before += wcount[piece][w];
-        const int64_t row = (int64_t)table[(int64_t)piece * nblocks + blockIdx.x] + before + __popc((is_own ? bo : bg) & lt);
-        send[3 * row] = x; send[3 * row + 1] = y; send[3 * row + 2] = z;
-        src_index[row] = i;
-    }
+    const unsigned lt = (1u << lane) - 1u;
+    for (int k = 0; k < R::kKinds; ++k)
+        for (int g = 0; g < a.world; ++g) {
+            const bool in = (m[k] >> g) & 1u;
+            const unsigned b = __ballot_sync(0xffffffffu, in);
+            if (!in) continue;
+            const int piece = k * a.world + g;
+            uint32_t before = 0;
+            for (int w = 0; w < warp; ++w) before += wcount[piece][w];
+            const int64_t row = (int64_t)table[(int64_t)piece * nblocks + blockIdx.x] + before + __popc(b & lt);
+            if (row < send_rows) a.put(send, src_index, row, i);
+            else *overflow = 1;
+        }
 }
 
-// counts[kind * world + g] = table entry of the first block of the NEXT piece - first block of this piece
+// counts[p] = table entry of the first block of the NEXT piece - first block of this piece
 __global__ void slab_route_counts_kernel(const uint64_t *__restrict__ table, const uint64_t *__restrict__ total, int64_t nblocks, int pieces,
                                          int64_t *__restrict__ counts)
 {
@@ -103,10 +156,57 @@ __global__ void slab_route_counts_kernel(const uint64_t *__restrict__ table, con
     counts[p] = (int64_t)(e - b);
 }
 
+static int64_t route_blocks(int64_t n) { return n > 0 ? (n + 255) / 256 : 1; }
+
+static size_t route_workspace(int pieces, int64_t n)
+{
+    const int64_t entries = (int64_t)pieces * route_blocks(n);
+    Carver c(nullptr);
+    c.take<uint64_t>(entries + 1);
+    c.take<char>(scan_workspace_bytes<uint64_t>(entries + 1));
+    return c.bytes();
+}
+
+// count pass + scan: counts[0 .. kKinds*world) and, in the workspace, the scanned block table (first send row of every
+// piece and block) that the write pass reads
+template <class R>
+static int route_count(const R &a, int64_t *counts, void *workspace, size_t workspace_bytes, cudaStream_t s)
+{
+    const int pieces = R::kKinds * a.world;
+    const size_t need = route_workspace(pieces, a.n);
+    if (!workspace || workspace_bytes < need) { set_error("workspace too small: need %zu bytes, have %zu", need, workspace_bytes); return AST_EWORKSPACE; }
+    const int64_t nb = route_blocks(a.n), entries = (int64_t)pieces * nb;
+    Carver c(workspace);
+    uint64_t *table = c.take<uint64_t>(entries + 1);
+    uint64_t *tmp = (uint64_t *)c.take<char>(scan_workspace_bytes<uint64_t>(entries + 1));
+    AST_CUDA_TRY(cudaMemsetAsync(table, 0, sizeof(uint64_t) * (entries + 1), s));
+    if (a.n > 0) slab_route_kernel<R, false><<<(unsigned)nb, 256, 0, s>>>(a, table, nb, nullptr, nullptr, 0, nullptr);
+    AST_KERNEL_CHECK(s, "slab_route_kernel<count>");
+    AST_CUDA_TRY(scan_exclusive<uint64_t>(table, entries, tmp, table + entries, s));      // total behind the table
+    slab_route_counts_kernel<<<1, 64, 0, s>>>(table, table + entries, nb, pieces, counts);
+    AST_KERNEL_CHECK(s, "slab_route_counts_kernel");
+    return AST_OK;
+}
+
+template <class R>
+static int route_write(const R &a, double *send, int64_t *src_index, int64_t send_rows, int *overflow, void *workspace,
+                       size_t workspace_bytes, cudaStream_t s)
+{
+    const size_t need = route_workspace(R::kKinds * a.world, a.n);
+    if (!workspace || workspace_bytes < need) { set_error("workspace too small: need %zu bytes, have %zu", need, workspace_bytes); return AST_EWORKSPACE; }
+    const int64_t nb = route_blocks(a.n);
+    Carver c(workspace);
+    uint64_t *table = c.take<uint64_t>((int64_t)R::kKinds * a.world * nb + 1);      // scanned by route_count on the same workspace
+    slab_route_kernel<R, true><<<(unsigned)nb, 256, 0, s>>>(a, table, nb, send, src_index, send_rows, overflow);
+    AST_KERNEL_CHECK(s, "slab_route_kernel<write>");
+    return AST_OK;
+}
+
 }  // namespace ast
 
 using namespace ast;
 
+// ---- k-NN exchange
 static int route_validate(const ast_slab_route_params *p)
 {
     AST_REQUIRE(p != nullptr, "params is null");
@@ -117,29 +217,23 @@ static int route_validate(const ast_slab_route_params *p)
     return AST_OK;
 }
 
-static int64_t route_blocks(int64_t n) { return n > 0 ? (n + 255) / 256 : 1; }
+static KnnRoute knn_route(const ast_slab_route_params *p, const double *pos, const int64_t *owner)
+{
+    KnnRoute a;
+    memset(&a, 0, sizeof a);
+    a.pos = pos; a.owner = owner; a.n = p->n; a.world = p->world; a.periodic = p->periodic; a.covers_all = p->covers_all;
+    a.length = p->length; a.w = p->w;
+    for (int g = 0; g < p->world; ++g) { a.b_lo[g] = p->bounds[g]; a.b_hi[g] = p->bounds[g + 1]; }
+    return a;
+}
 
 extern "C" int ast_slab_route_workspace_bytes(const ast_slab_route_params *p, size_t *bytes)
 {
     int rc = route_validate(p);
     if (rc) return rc;
     AST_REQUIRE(bytes != nullptr, "bytes is null");
-    const int64_t entries = 2 * (int64_t)p->world * route_blocks(p->n);
-    Carver c(nullptr);
-    c.take<uint64_t>(entries + 1);
-    c.take<char>(scan_workspace_bytes<uint64_t>(entries + 1));
-    *bytes = c.bytes();
+    *bytes = route_workspace(KnnRoute::kKinds * p->world, p->n);
     return AST_OK;
-}
-
-static RouteArgs route_args(const ast_slab_route_params *p, const double *pos, const int64_t *owner)
-{
-    RouteArgs a;
-    memset(&a, 0, sizeof a);
-    a.pos = pos; a.owner = owner; a.n = p->n; a.world = p->world; a.periodic = p->periodic; a.covers_all = p->covers_all;
-    a.length = p->length; a.w = p->w;
-    for (int g = 0; g < p->world; ++g) { a.b_lo[g] = p->bounds[g]; a.b_hi[g] = p->bounds[g + 1]; }
-    return a;
 }
 
 extern "C" int ast_slab_route_count(const ast_slab_route_params *p, const double *pos, const int64_t *owner, int64_t *counts,
@@ -148,22 +242,7 @@ extern "C" int ast_slab_route_count(const ast_slab_route_params *p, const double
     int rc = route_validate(p);
     if (rc) return rc;
     AST_REQUIRE(counts != nullptr && (p->n == 0 || (pos && owner)), "null pointer");
-    size_t need = 0;
-    ast_slab_route_workspace_bytes(p, &need);
-    if (!workspace || workspace_bytes < need) { set_error("workspace too small: need %zu bytes, have %zu", need, workspace_bytes); return AST_EWORKSPACE; }
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t nb = route_blocks(p->n), entries = 2 * (int64_t)p->world * nb;
-    Carver c(workspace);
-    uint64_t *table = c.take<uint64_t>(entries + 1);
-    uint64_t *tmp = (uint64_t *)c.take<char>(scan_workspace_bytes<uint64_t>(entries + 1));
-    RouteArgs a = route_args(p, pos, owner);
-    AST_CUDA_TRY(cudaMemsetAsync(table, 0, sizeof(uint64_t) * (entries + 1), s));
-    if (p->n > 0) slab_route_kernel<false><<<(unsigned)nb, 256, 0, s>>>(a, table, nb, nullptr, nullptr);
-    AST_KERNEL_CHECK(s, "slab_route_kernel<count>");
-    AST_CUDA_TRY(scan_exclusive<uint64_t>(table, entries, tmp, table + entries, s));      // total behind the table
-    slab_route_counts_kernel<<<1, 64, 0, s>>>(table, table + entries, nb, 2 * p->world, counts);
-    AST_KERNEL_CHECK(s, "slab_route_counts_kernel");
-    return AST_OK;
+    return route_count(knn_route(p, pos, owner), counts, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int ast_slab_route_write(const ast_slab_route_params *p, const double *pos, const int64_t *owner, double *send,
@@ -173,15 +252,68 @@ extern "C" int ast_slab_route_write(const ast_slab_route_params *p, const double
     if (rc) return rc;
     if (p->n == 0) return AST_OK;
     AST_REQUIRE(pos && owner && send && src_index, "null pointer");
-    size_t need = 0;
-    ast_slab_route_workspace_bytes(p, &need);
-    if (!workspace || workspace_bytes < need) { set_error("workspace too small: need %zu bytes, have %zu", need, workspace_bytes); return AST_EWORKSPACE; }
-    cudaStream_t s = (cudaStream_t)stream;
-    const int64_t nb = route_blocks(p->n);
-    Carver c(workspace);
-    uint64_t *table = c.take<uint64_t>(2 * (int64_t)p->world * nb + 1);      // scanned by ast_slab_route_count on the same workspace
-    RouteArgs a = route_args(p, pos, owner);
-    slab_route_kernel<true><<<(unsigned)nb, 256, 0, s>>>(a, table, nb, send, src_index);
-    AST_KERNEL_CHECK(s, "slab_route_kernel<write>");
+    // (this ABI has no row count: the caller allocates the counted total, so no row bound is passed)
+    return route_write(knn_route(p, pos, owner), send, src_index, INT64_MAX, nullptr, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- 3-D gridding on x-slabs
+static int grid_route_validate(const ast_grid_route_params *p)
+{
+    AST_REQUIRE(p != nullptr, "params is null");
+    AST_REQUIRE(p->n >= 0, "n < 0");
+    AST_REQUIRE(p->world >= 1 && p->world <= kRouteMaxWorld, "world = %d not in [1, %d]", p->world, kRouteMaxWorld);
+    AST_REQUIRE(p->nx > 0 && p->ny > 0 && p->nz > 0, "grid size must be positive");
+    for (int c = 0; c < 3; ++c) AST_REQUIRE(p->hi[c] > p->lo[c], "empty or inverted grid bounds");
+    if (p->periodic)
+        for (int c = 0; c < 3; ++c) AST_REQUIRE(p->box[c] > 0, "periodic routing needs box[0..2] > 0");
+    AST_REQUIRE(p->edges[0] >= 0 && p->edges[p->world] <= p->nx, "plane edges must lie in [0, nx = %d]", p->nx);
+    for (int g = 0; g < p->world; ++g) AST_REQUIRE(p->edges[g] <= p->edges[g + 1], "plane edges must not decrease");
     return AST_OK;
+}
+
+static GridRoute grid_route(const ast_grid_route_params *p, const double *pos, const double *h, const double *prop)
+{
+    GridRoute a;
+    memset(&a, 0, sizeof a);
+    a.pos = pos; a.h = h; a.prop = prop; a.n = p->n; a.world = p->world; a.periodic = p->periodic ? 1 : 0;
+    const int n3[3] = { p->nx, p->ny, p->nz };
+    for (int c = 0; c < 3; ++c) {
+        a.ax[c] = make_axis(p->lo[c], p->hi[c], n3[c]);
+        a.box[c] = p->periodic ? p->box[c] : 0.0;
+    }
+    for (int g = 0; g <= p->world; ++g) a.e[g] = p->edges[g];
+    return a;
+}
+
+extern "C" int ast_grid_route_workspace_bytes(const ast_grid_route_params *p, size_t *bytes)
+{
+    int rc = grid_route_validate(p);
+    if (rc) return rc;
+    AST_REQUIRE(bytes != nullptr, "bytes is null");
+    *bytes = route_workspace(GridRoute::kKinds * p->world, p->n);
+    return AST_OK;
+}
+
+extern "C" int ast_grid_route_count(const ast_grid_route_params *p, const double *pos, const double *h, int64_t *counts,
+                                    void *workspace, size_t workspace_bytes, void *stream)
+{
+    int rc = grid_route_validate(p);
+    if (rc) return rc;
+    AST_REQUIRE(counts != nullptr && (p->n == 0 || (pos && h)), "null pointer");
+    return route_count(grid_route(p, pos, h, nullptr), counts, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+extern "C" int ast_grid_route_write(const ast_grid_route_params *p, const double *pos, const double *h, const double *prop,
+                                    double *send, int64_t send_rows, int32_t *overflow, void *workspace, size_t workspace_bytes,
+                                    void *stream)
+{
+    int rc = grid_route_validate(p);
+    if (rc) return rc;
+    AST_REQUIRE(overflow != nullptr, "overflow is null");
+    AST_REQUIRE(send_rows >= 0 && (send_rows == 0 || send != nullptr), "send is null");
+    AST_REQUIRE(p->n == 0 || (pos && h && prop), "null pointer");
+    cudaStream_t s = (cudaStream_t)stream;
+    AST_CUDA_TRY(cudaMemsetAsync(overflow, 0, sizeof(int32_t), s));
+    if (p->n == 0) return AST_OK;
+    return route_write(grid_route(p, pos, h, prop), send, nullptr, send_rows, overflow, workspace, workspace_bytes, s);
 }

@@ -363,3 +363,227 @@ def smoothing_lengths_slabs(pos_local, k=32, box_size=None, group=None, solver=N
         return h_local, dict(iterations=iterations, ghost_width=w, ghost_fraction=(pos_slab.shape[0] - n_owned) / max(n_owned, 1),
                              owned=n_owned, local_set=int(pos_slab.shape[0]))
     return h_local
+
+
+# ---- 3-D gridding on x-slabs of the grid: each rank holds 1/G of the grid, particles go to the slabs their support reaches --
+def grid_slab_planes(nx, world):
+    """Plane edges e[0..world] of the x-slabs: rank g owns planes [e[g], e[g+1]) of an nx-plane grid.  Slabs are whole bricks
+    of 8 planes (the last one clipped to nx), split like shard_bounds, so every rank derives the same edges without a
+    collective; when nx < 8 * world the last ranks own no planes."""
+    nbx = -(-int(nx) // 8)
+    return [min(8 * shard_bounds(nbx, world, g)[0], int(nx)) for g in range(world)] + [int(nx)]
+
+
+def _check_route_inputs(pos, h, prop):
+    """the routing kernel reads pos[3 i], h[i], prop[i] through raw device pointers: anything but contiguous float64 CUDA
+    tensors of shapes (N, 3), (N,), (N,) on one device is refused before a launch"""
+    import torch
+    n = pos.shape[0] if isinstance(pos, torch.Tensor) and pos.dim() == 2 else -1
+    for name, t, shape in (("pos", pos, (n, 3)), ("h", h, (n,)), ("prop", prop, (n,))):
+        if not isinstance(t, torch.Tensor):
+            raise ValueError(f"grid routing: {name} must be a torch tensor")
+        if t.dtype != torch.float64 or tuple(t.shape) != shape or not t.is_cuda or not t.is_contiguous() or t.device != pos.device:
+            raise ValueError("grid routing needs contiguous float64 CUDA tensors on one device, pos (N,3), h (N,), prop (N,); "
+                             f"{name} is {t.dtype} {tuple(t.shape)} on {t.device}{'' if t.is_contiguous() else ', not contiguous'}")
+
+
+class _GridRouter:
+    """the routing kernel behind ast_grid_route_count / _write (csrc/slabroute.cu): two passes over the local particles"""
+
+    def __init__(self, device):
+        import threading
+        from . import _lib
+        import torch
+        self._lib = _lib
+        self.lib = _lib.load()
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        self.device = device
+        self._ws = None
+        self._lock = threading.RLock()        # one workspace: the count and the write pass of a call must not interleave with another's
+
+    def route(self, pos, h, prop, edges, grid_size, lo, hi, periodic, box):
+        """-> (send rows (S, 5) = x, y, z, h, prop [-> rank 0 | -> rank 1 | ...], counts per destination (world,) int64 on the
+        host, overflow flag (1,) int32 on the device: 1 if the write pass met a row beyond the counted total)"""
+        _check_route_inputs(pos, h, prop)
+        if pos.device != self.device:
+            raise ValueError(f"grid routing: tensors on {pos.device}, router on {self.device}")
+        with self._lock:
+            return self._route(pos, h, prop, edges, grid_size, lo, hi, periodic, box)
+
+    def _route(self, pos, h, prop, edges, grid_size, lo, hi, periodic, box):
+        import ctypes as C
+        import torch
+        _lib = self._lib
+        world = len(edges) - 1
+        p = _lib.GridRouteParams()
+        p.n = pos.shape[0]; p.world = world; p.periodic = 1 if periodic else 0
+        p.nx, p.ny, p.nz = (int(v) for v in grid_size)
+        b = (0.0, 0.0, 0.0)
+        if periodic:
+            b = (float(box),) * 3 if np.isscalar(box) else tuple(float(v) for v in box)
+        for c in range(3):
+            p.lo[c] = float(lo[c]); p.hi[c] = float(hi[c]); p.box[c] = b[c]
+        for g, e in enumerate(edges):
+            p.edges[g] = int(e)
+        need = C.c_size_t(0)
+        _lib.check(self.lib.ast_grid_route_workspace_bytes(C.byref(p), C.byref(need)))
+        if self._ws is None or self._ws.numel() < need.value:
+            self._ws = None
+            self._ws = torch.empty(need.value, dtype=torch.uint8, device=self.device)
+        stream = _lib.stream_ptr(None)
+        counts_d = torch.empty(world, dtype=torch.int64, device=self.device)
+        _lib.check(self.lib.ast_grid_route_count(C.byref(p), _lib.ptr(pos), _lib.ptr(h), _lib.ptr(counts_d), _lib.ptr(self._ws),
+                                                 C.c_size_t(self._ws.numel()), stream))
+        counts = counts_d.cpu()
+        total = int(counts.sum())
+        send = torch.empty((total, 5), dtype=torch.float64, device=self.device)
+        overflow = torch.empty(1, dtype=torch.int32, device=self.device)
+        _lib.check(self.lib.ast_grid_route_write(C.byref(p), _lib.ptr(pos), _lib.ptr(h), _lib.ptr(prop), _lib.ptr(send),
+                                                 C.c_int64(total), _lib.ptr(overflow), _lib.ptr(self._ws), C.c_size_t(self._ws.numel()),
+                                                 stream))
+        return send, counts, overflow
+
+
+_grid_routers = {}
+
+
+def default_grid_router(device):
+    """one _GridRouter (and its workspace) per device, reused by every grid_sharded call that injects none"""
+    import torch
+    device = torch.device(device)
+    key = torch.device(device.type, device.index if device.index is not None else torch.cuda.current_device())
+    if key not in _grid_routers:
+        _grid_routers[key] = _GridRouter(key)
+    return _grid_routers[key]
+
+
+def grid_sharded(gridder, pos, h, prop, grid_size, lo, hi, kernel="cubic_spline_3d", periodic=False, box=None, group=None,
+                 return_stats=False, router=None):
+    """Multi-GPU 3-D gridding without a full-size grid on any rank: rank r owns planes [e_r, e_{r+1}) of the grid
+    (grid_slab_planes) and gets back that slab, a (e_{r+1} - e_r, ny, nz) float64 tensor, with e_r: (slab, x_begin).
+    Every rank passes the particles it holds (any index range, any spatial spread):
+
+      1. the routing kernel sends every particle to each rank whose planes its support reaches (rows x, y, z, h, prop, in
+         ascending local index per destination);
+      2. ONE all-to-all of the per-destination row counts (the split sizes: one host synchronisation), each with the sender's
+         routing flag, so that if any rank's write pass met a row beyond its counted total every rank raises RuntimeError
+         here (that only happens through a bug; no rank enters the row exchange);
+      3. ONE all-to-all of the rows;
+      4. the rank grids what it received on its x window of the whole grid (gridder.grid(..., x_window=...)), whose voxel
+         corners are the whole grid's, bit for bit.
+
+    No collective is grid-sized.  `gridder` is a Gridder3D (or any object with its grid() signature) and `router` any object
+    with _GridRouter.route's signature: the CPU tests of this host logic inject oracle-backed stand-ins.  The default router
+    takes pos (N,3), h (N,), prop (N,) contiguous float64 CUDA tensors on one device and raises ValueError otherwise.  return_stats adds a
+    dict: rows sent to each rank, rows received, fan-out (rows sent / local particles) and the grid call's n_pairs / n_huge."""
+    import torch
+    import torch.distributed as dist
+    multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+    world, rank = (dist.get_world_size(group), dist.get_rank(group)) if multi else (1, 0)
+    nx, ny, nz = (int(v) for v in grid_size)
+    edges = grid_slab_planes(nx, world)
+    dev = pos.device
+    if router is None:
+        _check_route_inputs(pos, h, prop)
+        router = default_grid_router(dev)
+    send, counts, overflow = router.route(pos, h, prop, edges, grid_size, lo, hi, periodic, box)
+    counts = counts.to(torch.int64)
+    # row g = (rows for rank g, this rank's routing flag): after the exchange row g = (rows from rank g, rank g's flag)
+    flag = torch.zeros(1, dtype=torch.int64, device=dev) if overflow is None else overflow.to(device=dev, dtype=torch.int64)
+    out_d = torch.stack([counts.to(dev), flag.expand(world)], dim=1).contiguous()
+    if multi:
+        recv_d = torch.empty_like(out_d)
+        dist.all_to_all_single(recv_d, out_d, group=group)
+    else:
+        recv_d = out_d
+    host = recv_d.cpu()                                         # the split sizes and every rank's flag in one copy
+    recv = host[:, 0].tolist()
+    bad = [g for g in range(world) if host[g, 1]]
+    if bad:
+        raise RuntimeError(f"grid routing on rank(s) {bad} met a row beyond the counted total (count and write passes disagree)")
+    sent = counts.tolist()
+    if multi:
+        rows = torch.empty((sum(recv), 5), dtype=torch.float64, device=dev)
+        dist.all_to_all_single(rows, send, output_split_sizes=recv, input_split_sizes=sent, group=group)
+    else:
+        rows = send
+    del send
+    x0, x1 = edges[rank], edges[rank + 1]
+    stats = None
+    if x1 > x0:
+        slab = gridder.grid(rows[:, :3].contiguous(), rows[:, 3].contiguous(), rows[:, 4].contiguous(), grid_size, lo, hi, kernel,
+                            periodic, box, x_window=(x0, x1))
+        stats = getattr(gridder, "last_stats", None)
+    else:
+        slab = torch.zeros((0, ny, nz), dtype=torch.float64, device=dev)
+    if return_stats:
+        st = dict(sent=sent, received=sum(recv), fan_out=sum(sent) / max(pos.shape[0], 1), x_begin=x0, x_end=x1,
+                  n_pairs=stats["n_pairs"] if stats else 0, n_huge=stats["n_huge"] if stats else 0)
+        return slab, x0, st
+    return slab, x0
+
+
+def collect_slabs(slab, nx, dst=0, group=None, all_ranks=False):
+    """The whole (nx, ny, nz) grid from the x-slabs of grid_sharded, on `dst` (or every rank); None elsewhere.  Slabs are
+    contiguous plane blocks of the C-order grid, so collecting them on dst is one all-to-all whose only non-empty splits go
+    to dst, with no reorder.  all_ranks all-gathers the slabs, padded to the thickest, straight into one buffer of
+    world * thickest planes (at most 8 * world planes more than the grid) and moves each slab down to its planes in place,
+    so a rank holds one grid, not a gathered copy plus a concatenation."""
+    import torch
+    import torch.distributed as dist
+    if not (dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1):
+        return slab
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    edges = grid_slab_planes(nx, world)
+    planes = [edges[g + 1] - edges[g] for g in range(world)]
+    if all_ranks:
+        tp = max(planes)
+        buf = torch.empty((world * tp,) + tuple(slab.shape[1:]), dtype=slab.dtype, device=slab.device)
+        mine = slab.contiguous()
+        if planes[rank] < tp:
+            mine = torch.zeros((tp,) + tuple(slab.shape[1:]), dtype=slab.dtype, device=slab.device)
+            mine[:planes[rank]] = slab
+        dist.all_gather([buf[g * tp:(g + 1) * tp] for g in range(world)], mine, group=group)
+        # slab g sits at g * tp and belongs at edges[g] <= g * tp: move it down in blocks no longer than the shift, in
+        # ascending order, so that no block overwrites planes not yet moved
+        for g in range(1, world):
+            src, dst, shift = g * tp, edges[g], g * tp - edges[g]
+            for k in range(0, planes[g] if shift else 0, max(shift, 1)):
+                m = min(shift, planes[g] - k)
+                buf[dst + k:dst + k + m].copy_(buf[src + k:src + k + m])
+        return buf[:nx]
+    send_splits = [planes[rank] if g == dst else 0 for g in range(world)]
+    recv_splits = planes if rank == dst else [0] * world
+    whole = torch.empty((sum(recv_splits),) + tuple(slab.shape[1:]), dtype=slab.dtype, device=slab.device)
+    dist.all_to_all_single(whole, slab.contiguous(), output_split_sizes=recv_splits, input_split_sizes=send_splits, group=group)
+    return whole if rank == dst else None
+
+
+def create_grid_sharded(positions, smoothing_lengths, particle_properties, grid_size, x_min, x_max, y_min, y_max, z_min, z_max,
+                        kernel_func=None, *, periodic=False, box_size=None, dst=0, group=None, all_ranks=False):
+    """Host-buffer entry for one rank of a multi-GPU job: create_grid's arguments, but the arrays hold only THIS rank's
+    particles.  Each rank grids its x-slab (grid_sharded); the slabs are collected on `dst` (or on every rank) and the
+    whole (nx, ny, nz) float64 numpy grid is returned there, None elsewhere.  kernel_func=None is quartic_spline_kernel."""
+    import torch
+    from .tools.projections._gridder import default_gridder
+    from .tools.projections._kernels import kernel_id_of, quartic_spline_kernel
+    from .tools.projections._projector import _check_buffer
+    kernel = kernel_id_of(kernel_func if kernel_func is not None else quartic_spline_kernel)
+    positions = _check_buffer(positions, 2, "positions")
+    smoothing_lengths = _check_buffer(smoothing_lengths, 1, "smoothing_lengths")
+    particle_properties = _check_buffer(particle_properties, 1, "particle_properties")
+    if positions.shape[1] != 3 or not (positions.shape[0] == smoothing_lengths.shape[0] == particle_properties.shape[0]):
+        raise ValueError("positions (N,3), smoothing_lengths (N,), particle_properties (N,) expected")
+    eng = default_gridder()
+    to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a)).to(eng.device)
+    nx, ny, nz = (int(v) for v in grid_size)
+    slab, _ = grid_sharded(eng, to_dev(positions), to_dev(smoothing_lengths), to_dev(particle_properties), (nx, ny, nz),
+                           (x_min, y_min, z_min), (x_max, y_max, z_max), kernel, periodic, box_size, group)
+    whole = collect_slabs(slab, nx, dst, group, all_ranks)
+    if whole is not None:
+        host = torch.empty(whole.shape, dtype=whole.dtype, pin_memory=whole.is_cuda)
+        host.copy_(whole)
+        return host.numpy()
+    return None

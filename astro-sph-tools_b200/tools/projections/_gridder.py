@@ -29,10 +29,14 @@ class Gridder3D:
         self.last_stats = None
         self._lock = threading.RLock()        # one workspace: calls on this engine serialise
 
-    def params(self, n, grid_size, lo, hi, kernel, periodic=False, box=None, timing=False, accumulate=False):
+    def params(self, n, grid_size, lo, hi, kernel, periodic=False, box=None, timing=False, accumulate=False, x_window=None):
         p = _lib.Grid3DParams()
         p.n = int(n)
         p.nx, p.ny, p.nz = (int(v) for v in grid_size)
+        if x_window is not None:
+            p.x_begin, p.x_end = (int(v) for v in x_window)
+            if not 0 <= p.x_begin < p.x_end <= p.nx:
+                raise ValueError(f"x_window {tuple(x_window)} is not inside [0, {p.nx})")
         if isinstance(kernel, str):
             p.kernel_id = _lib.KERNEL_IDS[kernel]
         elif hasattr(kernel, "device_table"):                      # TabulatedKernel: arbitrary kernel_func callable
@@ -72,14 +76,16 @@ class Gridder3D:
         return self._ws
 
     def grid(self, pos, h, prop, grid_size, lo, hi, kernel="cubic_spline_3d", periodic=False, box=None, out=None, timing=False,
-             accumulate=False, stream=None, presort="auto"):
-        """pos (N,3), h (N,), prop (N,) float64 CUDA tensors -> (nx,ny,nz) float64 CUDA tensor"""
+             accumulate=False, stream=None, presort="auto", x_window=None):
+        """pos (N,3), h (N,), prop (N,) float64 CUDA tensors -> (nx,ny,nz) float64 CUDA tensor.
+        x_window=(x_begin, x_end): planes [x_begin, x_end) of that grid only, a (x_end - x_begin, ny, nz) tensor whose voxels
+        are bit for bit the whole grid's voxel corners (so a slab has the same contributors as in the whole grid)."""
         torch = self.torch
         n = pos.shape[0]
         for t, shape in ((pos, (n, 3)), (h, (n,)), (prop, (n,))):
             if t.dtype != torch.float64 or tuple(t.shape) != shape or not t.is_cuda or not t.is_contiguous():
                 raise ValueError("device inputs must be contiguous float64 CUDA tensors of shapes (N,3), (N,), (N,)")
-        p = self.params(n, grid_size, lo, hi, kernel, periodic, box, timing, accumulate)
+        p = self.params(n, grid_size, lo, hi, kernel, periodic, box, timing, accumulate, x_window)
         # optional spatial pre-ordering: 'auto' = the library looks at a sample of the input order (the deposition is 27 % faster
         # on the randomly ordered NFW set of config 4 when the particles are first ordered by brick), 'always', 'never'
         if presort in (True, "always"):
@@ -89,7 +95,7 @@ class Gridder3D:
         elif presort not in (None, False, "never"):
             raise ValueError("presort must be 'auto', 'always' or 'never'")
         if out is None:
-            out = torch.empty((p.nx, p.ny, p.nz), dtype=torch.float64, device=self.device)
+            out = torch.empty((p.x_end - p.x_begin if x_window is not None else p.nx, p.ny, p.nz), dtype=torch.float64, device=self.device)
         stats = _lib.Project2DStats()
         with torch.cuda.device(self.device), self._lock:
             # pair_capacity / huge_capacity are windows (the library walks any number of pairs and large-h entries through them

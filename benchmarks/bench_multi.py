@@ -4,6 +4,9 @@
                (STRONG scaling: total work fixed), NCCL sum-reduce of the partial maps
   --which c5   config 5 slice: k-NN k=48 periodic on n^3 particles; positions replicated on every rank (generated on the
                device from a fixed seed), rank g answers queries [g*N/G, (g+1)*N/G)
+  --which c4   config 4: 256^3 NFW-clustered particles -> 512^3 voxels, periodic, through distributed.grid_sharded: particles
+               sharded by index, each rank owns one x-slab of the grid (1/G of it); parity on a 48^3 window of the assembled
+               grid against the float64 oracle, as in bench.py's c4 sub-record
 Rank 0 prints one JSON object per configuration.  Timing: CUDA events, barrier + synchronize on both sides, max over ranks."""
 import argparse
 import json
@@ -97,8 +100,63 @@ def main():
                                         f"NCCL reduce", "ms": ms, "particles_per_s": N / (ms * 1e-3), "n_gpus": world, "scaling": "strong",
                               "hbm_frac_vs_one_gpu_roofline": alg / (ms * 1e-3) / 1e9 / peak, "sum_img_times_pixel_area": total,
                               "pairs_rank0": eng.last_stats["n_pairs"]}))
+    if "c4" in args.which:
+        c4(torch, dist, astd, dev, world, rank, timed, sync)
     if world > 1:
         dist.destroy_process_group()
+
+
+def c4(torch, dist, astd, dev, world, rank, timed, sync):
+    import oracle
+    from bench import nfw_positions_device, parity_of
+    from astro_sph_tools_b200.tools.projections import Gridder3D
+    from astro_sph_tools_b200.tools.smoothing import SmoothingLengthSolver
+    n, ng = 256, 512
+    N = n ** 3
+    size, lo, hi = (ng,) * 3, (0.0, 0.0, 0.0), (1.0, 1.0, 1.0)
+    pos = nfw_positions_device(torch, dev, N)                  # the same set on every rank (fixed seed)
+    sol = SmoothingLengthSolver(device=dev)
+    h = sol.solve(pos, 48, 1.0)
+    sol._ws = None
+    torch.cuda.empty_cache()
+    a, b = astd.shard_bounds(N, world, rank)
+    pos_l, h_l = pos[a:b].contiguous(), h[a:b].contiguous()
+    m_l = torch.full((b - a,), 1.0 / N, dtype=torch.float64, device=dev)
+    g = Gridder3D(device=dev)
+    router = astd.default_grid_router(dev)
+    edges = astd.grid_slab_planes(ng, world)
+    route_ms = timed(lambda: router.route(pos_l, h_l, m_l, edges, size, lo, hi, True, 1.0), 3)
+    e8 = astd.grid_slab_planes(ng, 8)                          # routing (count + write) of this rank's particles into 8 slabs
+    route8_ms = timed(lambda: router.route(pos_l, h_l, m_l, e8, size, lo, hi, True, 1.0), 3)
+    out = {}
+    step = lambda: out.__setitem__("r", astd.grid_sharded(g, pos_l, h_l, m_l, size, lo, hi, periodic=True, box=1.0, return_stats=True))
+    ms = timed(step, 3)
+    slab, x0, st = out["r"]
+    loads = torch.tensor([[float(st["n_pairs"]), float(st["received"]), float(sum(st["sent"]))]], dtype=torch.float64, device=dev)
+    parts = [torch.zeros_like(loads) for _ in range(world)]
+    if world > 1:
+        dist.all_gather(parts, loads)
+    else:
+        parts = [loads]
+    loads = torch.cat(parts).cpu().numpy()
+    rec = {"config": f"C4: S2 NFW {n}^3 = {N} particles -> {ng}^3 voxels, periodic, grid_sharded over {world} GPU(s), x-slabs of "
+                     f"{ng // world if ng % world == 0 else 'about ' + str(ng // world)} planes",
+           "ms": ms, "route_ms_rank0": route_ms, "route_into_8_slabs_ms_rank0": route8_ms, "n_gpus": world, "fan_out": float(loads[:, 2].sum() / N),
+           "n_pairs_max": float(loads[:, 0].max()), "n_pairs_mean": float(loads[:, 0].mean()), "rows_received_max": float(loads[:, 1].max())}
+    if world == 1:
+        whole = torch.empty(size, dtype=torch.float64, device=dev)
+        rec["gridder3d_ms"] = timed(lambda: g.grid(pos, h, m_l, size, lo, hi, periodic=True, box=1.0, out=whole), 3)
+    whole = astd.collect_slabs(slab, ng, dst=0)
+    if rank == 0:
+        wv, v0 = 48, ng // 2 - 24
+        wlo, whi = v0 / ng, (v0 + wv) / ng
+        p, hh = pos.cpu().numpy(), h.cpu().numpy()
+        sel = np.all((p + 2.0 * hh[:, None] > wlo) & (p - 2.0 * hh[:, None] < whi), axis=1)
+        ref = oracle.grid3d(p[sel], hh[sel], np.full(int(sel.sum()), 1.0 / N), (wv,) * 3, (wlo,) * 3, (whi,) * 3)
+        crop = whole[v0:v0 + wv, v0:v0 + wv, v0:v0 + wv].cpu().numpy()
+        rec["parity"] = dict(parity_of(crop, ref), window=f"{wv}^3 voxels at [{wlo:g},{whi:g})^3")
+        print(json.dumps(rec), flush=True)
+    sync()
 
 
 if __name__ == "__main__":

@@ -162,6 +162,12 @@ typedef struct ast_grid3d_params {
     const float *kernel_table;   /* as in ast_project2d_params */
     int32_t kernel_table_n;
     int32_t kernel_dim;
+    /* x window: compute planes [x_begin, x_end) of the nx-plane grid only; out holds (x_end - x_begin)*ny*nz doubles,
+     * plane x_begin first.  0, 0 = the whole grid.  Every voxel corner is the whole grid's (lo[0] + (x_begin + i)*d, d =
+     * (hi[0] - lo[0])/nx), so a window's voxels have the same contributors, bit for bit, as in the whole-grid call; bricks
+     * and bboxes are numbered from x_begin.  AST_EINVAL unless 0 <= x_begin < x_end <= nx (or both 0).  Appended at the
+     * end of the struct: every earlier field keeps its offset, so the ABI version is unchanged. */
+    int32_t x_begin, x_end;
 } ast_grid3d_params;
 
 int ast_grid3d_workspace_bytes(const ast_grid3d_params *p, size_t *bytes);
@@ -172,7 +178,9 @@ int ast_grid3d(const ast_grid3d_params *p, const double *pos, const double *h, c
  * pairs_sorted pair_capacity uint64 = (sort_key << 32) | particle with sort_key = brick_key * (periodic ? 32 : 1) + image,
  * brick_key = (bx*nby + by)*nbz + bz, sorted (stably) by brick_key only; the tiled pairs are followed by the member bricks
  * of the large-h entries (list order; bx, by, bz ascending); huge = (image << 32) | particle; counts (host) = {pairs (large-h
- * pairs included), large-h entries}.  Here the capacities are limits.  Synchronises. */
+ * pairs included), large-h entries}.  Here the capacities are limits.  Synchronises.  With an x window the bboxes are the
+ * whole grid's clipped to the window and shifted by -x_begin (empty when the x range misses the window), and classes,
+ * pairs and the large-h list follow from those bboxes and the window's bricks. */
 int ast_bin3d(const ast_grid3d_params *p, const double *pos, const double *h, int32_t *bbox, uint8_t *cls,
               uint64_t *pairs_sorted, uint64_t *huge, int64_t *counts, void *workspace, size_t workspace_bytes,
               void *stream);
@@ -271,6 +279,29 @@ int ast_slab_route_count(const ast_slab_route_params *p, const double *pos, cons
                          void *workspace, size_t workspace_bytes, void *stream);
 int ast_slab_route_write(const ast_slab_route_params *p, const double *pos, const int64_t *owner, double *send,
                          int64_t *src_index, void *workspace, size_t workspace_bytes, void *stream);
+
+/* ---- multi-GPU 3-D gridding: routing of particles to x-slabs of the grid.  Rank g owns planes [e[g], e[g+1]) of the
+ * whole grid (lo, hi, nx, ny, nz; box when periodic); particle i goes to rank g iff some periodic image of it (the particle
+ * itself when not periodic) has a non-empty contributor range on the whole grid's x axis that meets [e[g], e[g+1]), and
+ * some image has a non-empty range on y and on z: exactly the particles that ast_grid3d with that x window would deposit
+ * (same ranges, same float64 arithmetic).  ast_grid_route_count fills counts[0..world) (device, int64) and leaves the
+ * scanned block table in the workspace; ast_grid_route_write (same params, same workspace, after the count) writes rows
+ * (x, y, z, h, prop) of 5 doubles, [-> rank 0 | -> rank 1 | ...], ascending particle index inside each piece.  send_rows
+ * is the number of rows `send` holds (the counted total): a row beyond it is not written and sets *overflow (device int32,
+ * zeroed by the call) to 1. */
+typedef struct ast_grid_route_params {
+    int64_t n;
+    int32_t world, periodic;
+    int32_t nx, ny, nz, reserved;
+    double lo[3], hi[3], box[3];
+    int32_t edges[AST_ROUTE_MAX_WORLD + 1];   /* plane edges e[0..world], non-decreasing, e[0] >= 0, e[world] <= nx */
+} ast_grid_route_params;
+int ast_grid_route_workspace_bytes(const ast_grid_route_params *p, size_t *bytes);
+int ast_grid_route_count(const ast_grid_route_params *p, const double *pos, const double *h, int64_t *counts,
+                         void *workspace, size_t workspace_bytes, void *stream);
+int ast_grid_route_write(const ast_grid_route_params *p, const double *pos, const double *h, const double *prop,
+                         double *send, int64_t send_rows, int32_t *overflow, void *workspace, size_t workspace_bytes,
+                         void *stream);
 
 /* ---- misc ---- */
 const char *ast_last_error(void);
